@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            (this framework, CUDA)
   python bench.py --impl reference --gpus N --steps K ...  (the reference's algorithm on
                                                             the host CPU cores: oracle port)
+  python bench.py ... --dump-outputs DIR                    (also write the last timed step's outputs
+                                                            as DIR/<name>.npy)
 Under torchrun (N > 1) every rank runs one learner replica on its own GPU (batch-axis
 sharding, B=64 unrolls per GPU) with ONE NCCL all-reduce(SUM) of the flat gradient arena
 per step; the timed region is bracketed by barrier + synchronize, timed with CUDA events,
@@ -52,7 +54,14 @@ def parse_args():
                       "operand planes with TMA-fed warp-specialised kernels (deep net; the default)")
   p.add_argument('--no-extras', action='store_true',
                  help='skip the profiling pass, the loss-kernel sweep and the CPU baseline')
+  p.add_argument('--dump-outputs', metavar='DIR',
+                 help='after the timed steps, write what the last timed step computed (loss terms, updated '
+                      'parameters, gradients; R2D2 also priorities and sampled indices) as DIR/<name>.npy')
   a = p.parse_args()
+  if a.steps < 1:
+    p.error('--steps must be at least 1')
+  if a.dump_outputs and a.impl == 'reference':
+    p.error('--dump-outputs writes the outputs of the CUDA path (--impl b200)')
   if a.net == 'shallow' and a.conv == 'tc3p':
     a.conv = 'tc3'
   if a.cpu_batch <= 0:
@@ -500,12 +509,15 @@ def run_r2d2(args):
   while not feeder.ready() or replay.num_inserted < st.replay_buffer_size:
     feeder.insert(dev_new)
 
+  last_step = [None]
+
   def one_step(from_host):
     new = utils.map_structure(lambda t: t.cuda(non_blocking=True), host_new) if from_host else dev_new
     feeder.insert(new)
     sampled = feeder.sample()
     loss, priorities, indices, norm = step.minimize(sampled)
     feeder.update_priorities(indices, priorities)
+    last_step[0] = (loss, priorities, indices, norm)
     return loss
 
   def timed(fn, k):
@@ -526,6 +538,12 @@ def run_r2d2(args):
   launches = (_lib.launch_count() - n0) // args.steps
   agent.check_errors()
   clocks = sampler.stop()
+  if args.dump_outputs:
+    loss, priorities, indices, norm = last_step[0]
+    outputs = {'loss': loss, 'priorities': priorities, 'indices': indices, 'gradient_norm': norm}
+    outputs.update(('param/' + k, v) for k, v in agent.named_parameters().items())
+    outputs.update(('grad/' + k, v) for k, v in agent.named_gradients().items())
+    dump_outputs(args.dump_outputs, outputs)
   ms_e2e = timed(lambda: float(one_step(True)), args.steps)
   frames = B * st.unroll_length
   line = {'metric': R2D2_METRIC, 'value': frames / (ms * 1e-3), 'unit': UNIT, 'n_gpus': 1, 'steps': args.steps,
@@ -587,6 +605,26 @@ def r2d2_gemm_flops(T, B, burn_in):
   fwd = 2 * T * B * per_frame
   bwd = 2 * (T - burn_in) * B * per_frame
   return 2 * (fwd + bwd)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+  """Writes every tensor of `arrays` as path/<name>.npy ('/' in a name becomes '.'): floating point as
+  float32 (float64 stays float64), integers as float64 (exact below 2**53), so that two builds can be
+  compared file by file."""
+  import numpy as np
+  out = {}
+  for name, t in arrays.items():
+    a = t.detach().cpu().numpy()
+    out[name.replace('/', '.')] = a.astype(np.float32 if a.dtype.kind == 'f' and a.itemsize <= 4 else np.float64)
+  total = sum(a.nbytes for a in out.values())
+  if total > DUMP_LIMIT_BYTES:
+    raise SystemExit('bench.py: --dump-outputs would write %d bytes, more than %d' % (total, DUMP_LIMIT_BYTES))
+  os.makedirs(path, exist_ok=True)
+  for name, a in out.items():
+    np.save(os.path.join(path, name + '.npy'), a)
 
 
 _JSON_FD = None
@@ -705,6 +743,13 @@ def main():
   ms_step_median = last_median[0]
   agent.check_errors()      # raises if any kernel of the timed steps timed out on a barrier
   clocks = sampler.stop() if sampler else None
+  if args.dump_outputs and rank == 0:
+    # the last timed step's loss terms (the loss `minimize` returned is 'total') and the state it left
+    outputs = {'loss/' + k: step.last_loss_terms[i] for k, i in _lib.LT.items()}
+    outputs.update(('param/' + k, v) for k, v in agent.named_parameters().items())
+    outputs['param/entropy_cost_param'] = agent.entropy_cost_param
+    outputs.update(('grad/' + k, v) for k, v in agent.named_gradients().items())
+    dump_outputs(args.dump_outputs, outputs)
   value = world * B * T / (ms_step * 1e-3)
 
   # ---- end to end: pinned host batch -> H2D -> step -> loss to host ---------------------
