@@ -180,9 +180,9 @@ size_t seedrl_net_arena_floats(const seedrl_net* net);
  * format): TMA-fed, warp-specialised conv kernels (csrc/conv_planes.cu; deep net only). */
 int seedrl_net_set_conv_mode(seedrl_net* net, int mode);
 /* LSTM recurrence: 2 (default) = one persistent kernel for all T steps each way with CTA = (batch
- * tile, 16 hidden units) and one barrier counter per batch tile (csrc/lstm_tiled.cu); 1 = the first
- * persistent form, CTA = 2 hidden units x all rows, one grid barrier per step (csrc/lstm_persistent.cu);
- * 0 = a GEMM + a pointwise kernel per time step. */
+ * tile, 16 hidden units) and one barrier counter per batch tile (csrc/lstm_tiled.cu); 0 = a GEMM + a
+ * pointwise kernel per time step (the reference the tiled kernels are tested against).  1 (an earlier
+ * persistent form, since removed) is rejected with SEEDRL_ERR_INVALID_ARGUMENT. */
 int seedrl_net_set_lstm_mode(seedrl_net* net, int mode);
 /* name is written into buf (NUL-terminated); shape into dims[0..3], rank returned. */
 int seedrl_net_param_info(const seedrl_net* net, int index, char* name_buf,
@@ -354,7 +354,7 @@ int seedrl_r2d2_net_num_param_tensors(const seedrl_r2d2_net* net);      /* 18 */
 size_t seedrl_r2d2_net_num_params(const seedrl_r2d2_net* net);
 size_t seedrl_r2d2_net_arena_floats(const seedrl_r2d2_net* net);
 int seedrl_r2d2_net_set_mode(seedrl_r2d2_net* net, int mode);
-int seedrl_r2d2_net_set_lstm_mode(seedrl_r2d2_net* net, int mode);   /* as seedrl_net_set_lstm_mode: 1 or 2 */
+int seedrl_r2d2_net_set_lstm_mode(seedrl_r2d2_net* net, int mode);   /* as seedrl_net_set_lstm_mode: 0 or 2 */
 int seedrl_r2d2_net_param_info(const seedrl_r2d2_net* net, int index, char* name_buf, size_t name_buf_len,
                                int64_t* dims4, int* rank, size_t* offset_floats);
 size_t seedrl_r2d2_net_workspace_bytes(const seedrl_r2d2_net* net, int T, int B);

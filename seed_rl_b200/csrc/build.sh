@@ -4,7 +4,7 @@ set -e
 cd "$(dirname "$0")"
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 OUT=../libseedrl_b200.so
-SRCS="capi.cu vtrace_kernels.cu r2d2_kernels.cu optim_kernels.cu conv_kernels.cu conv_tc_kernels.cu conv_planes.cu conv_first.cu convgen_kernels.cu gemm_kernels.cu gemm_tc_kernels.cu lstm_persistent.cu lstm_tiled.cu net.cu r2d2_net.cu store_kernels.cu batcher.cc"
+SRCS="capi.cu vtrace_kernels.cu r2d2_kernels.cu optim_kernels.cu conv_kernels.cu conv_tc_kernels.cu conv_planes.cu conv_first.cu convgen_kernels.cu gemm_kernels.cu gemm_tc_kernels.cu lstm_tiled.cu net_common.cu net.cu r2d2_net.cu store_kernels.cu batcher.cc"
 mkdir -p build
 OBJS=""
 pids=""

@@ -1,5 +1,8 @@
 // Internal host-side launchers shared between translation units.
 #pragma once
+#include <initializer_list>
+#include <vector>
+
 #include "common.cuh"
 
 namespace seedrl {
@@ -155,11 +158,6 @@ int convgen_wgrad(int N, int H, int W, int cin, int cout, int k, int stride, int
                   const void* x, const float* dy, float* dw, float* db, float* partial,
                   size_t partial_bytes, cudaStream_t st);
 
-// r2d2_net.cu: 'valid' strided convolutions as im2col + GEMM (R2D2 body, shallow IMPALA net)
-int im2col_nhwc(int N, int H, int W, int C, int K, int S, int in_u8, const void* x, float* col, cudaStream_t st);
-int col2im_nhwc(int N, int H, int W, int C, int K, int S, const float* dcol, const float* xmask, float* dx,
-                cudaStream_t st);
-
 // gemm_kernels.cu
 struct GemmEpi {
   const float* bias;
@@ -214,20 +212,103 @@ int lstm_pointwise_bwd(int B, int Hd, const float* gates, const float* c_t, cons
                        cudaStream_t st);
 int fill(size_t n, float* p, float v, cudaStream_t st);
 
-// lstm_persistent.cu (H = 256: ImpalaDeep core; H = 512: DuelingLSTMDQNNet core)
-int lstm_forward_persistent(int H, int T1, int B, const float* U, const uint8_t* done, float* z,
-                            const float* h0, const float* c0, float* hs, float* cs, float* hp,
-                            unsigned int* counter, int* err, cudaStream_t st);
-int lstm_backward_persistent(int H, int T1, int B, const float* U, const uint8_t* done, const float* gates,
-                             const float* cs, const float* c0, const float* dhs, float* dz,
-                             unsigned int* counter, int* err, cudaStream_t st);
-
-// lstm_tiled.cu: CTA = (batch tile, 16 hidden units), one barrier counter per batch tile
+// lstm_tiled.cu (H = 256: ImpalaDeep core; H = 512: DuelingLSTMDQNNet core): CTA = (batch tile, 16
+// hidden units), one barrier counter per batch tile
 int lstm_forward_tiled(int H, int T1, int B, const float* U, const uint8_t* done, float* z, const float* h0,
                        const float* c0, float* hs, float* cs, float* hp, unsigned int* counter, int* err,
                        cudaStream_t st);
 int lstm_backward_tiled(int H, int T1, int B, const float* U, const uint8_t* done, const float* gates,
                         const float* cs, const float* c0, const float* dhs, float* dz, unsigned int* counter,
                         int* err, cudaStream_t st);
+
+// ---- net_common.cu: host-side pieces of the two network schedules (net.cu, r2d2_net.cu) ----------
+
+// Parameter table of one flat fp32 arena: tensors in creation order, every start aligned to 64 floats
+// (256 B).
+struct ParamInfo {
+  std::string name;
+  int rank;
+  int64_t dims[4];   // trailing dims beyond the rank are 1
+  size_t offset;     // floats
+  size_t size;       // floats
+};
+struct ParamTable {
+  std::vector<ParamInfo> params;
+  size_t arena_floats = 0;
+  int add(const std::string& name, std::initializer_list<int64_t> dims);   // returns the tensor's index
+  // Copies the name (NUL-terminated, truncated to name_buf_len), dims[0..3] and offset of tensor
+  // `index`, each when its pointer is non-null; returns the rank, or -1 for an index out of range.
+  int info(int index, char* name_buf, size_t name_buf_len, int64_t* dims, size_t* offset) const;
+  template <typename T>
+  T* at(T* arena, int idx) const { return arena + params[idx].offset; }
+};
+
+// Workspace plan: consecutive 256-byte aligned offsets, and the typed pointer at one of them.
+struct Bump {
+  size_t off = 0;
+  size_t take(size_t bytes);
+};
+template <typename T>
+inline T* W(void* ws, size_t off) {
+  return reinterpret_cast<T*>(reinterpret_cast<char*>(ws) + off);
+}
+
+// The dense contractions of a schedule: tcgen05 when `tc` is set and the shape is worth a 128-row
+// tile (gemm_tc_supported), else the fp32 SIMT kernel.  `ws` holds the split-K partials
+// (gemm_tc_workspace_bytes()); *err is set when a bounded barrier wait expires.
+struct GemmRunner {
+  bool tc;
+  int split;        // bf16x3 operands
+  float* ws;
+  int* err;
+  int gemm(bool ta, bool tb, int M, int N, int K, const float* A, int lda, const float* B, int ldb, float* C,
+           int ldc, const GemmEpi& e, cudaStream_t st) const;
+  // op(A) = the gathered im2col matrix `cg` (tcgen05 only, see gemm_tc)
+  int gemm_gather(bool ta, int M, int N, int K, const ConvGather& cg, const float* B, int ldb, float* C, int ldc,
+                  const GemmEpi& e, cudaStream_t st) const;
+  // bias gradient: out[n] = sum_m X[m*ld + n], with `ws` as the row-slab scratch
+  int colsum(int M, int N, const float* X, int ld, float* out, cudaStream_t st) const;
+};
+
+// Reads back the error flag the tcgen05 / persistent kernels of the last forward/backward set when a
+// bounded barrier wait expired (their results are then garbage).  Synchronises `st`.
+int read_error_flag(const int* flag, cudaStream_t st);
+
+// A 'valid' k x k / stride s convolution of NHWC tensors as a GEMM over its im2col matrix (rows =
+// output positions (n, ho, wo), columns = (kh, kw, c)); Keras HWIO weights = [k*k*cin, cout].
+struct StridedConv { int k, s, cin, cout, hin, win, hout, wout, w, b; };   // w, b: parameter indices
+StridedConv strided_conv(int k, int s, int cin, int cout, int hin, int win);
+// y = relu(im2col(x) W + b).  The im2col matrix is gathered inside the GEMM where the geometry allows
+// it, else materialised in `col` and kept there for the backward.  u8: x holds uint8 frames, scaled
+// by 1/255.
+int strided_conv_forward(const GemmRunner& g, int N, const StridedConv& c, bool u8, const void* x, const float* w,
+                         const float* bias, float* col, float* y, cudaStream_t st);
+// dW = im2col(x)^T dy (gathered from x, or from the matrix the forward kept in `col`), db = column sums
+// of dy; with dx (x = the ReLU'd fp32 activation): dcol = dy W^T written over `col`, dx = col2im(dcol)
+// masked by x > 0.
+int strided_conv_backward(const GemmRunner& g, int N, const StridedConv& c, bool u8, const void* x, float* col,
+                          const float* w, const float* dy, float* dw, float* db, float* dx, cudaStream_t st);
+
+// Keras LSTMCell(H) over T1 steps with done-resets, on N = T1 * B rows: the input projection of all
+// steps as one GEMM, then the recurrence as the tiled kernels (lstm_tiled.cu) or, as their reference,
+// a GEMM + a pointwise kernel per step.  Workspace offsets of its buffers:
+//   xc [N, CI] core input (filled by the net), z / dz [N, 4H] gates, hp [N, H] masked h(t-1),
+//   cs / hs / dhs / dd [N, H], c0buf / dhrec / dc0 / dc1 [B, H].
+struct LstmBufs { size_t xc, z, hp, cs, hs, c0buf, dhs, dz, dhrec, dc0, dc1, dd; };
+LstmBufs lstm_bufs(Bump* b, size_t N, int B, int H, int CI);
+struct LstmCore {
+  int H, CI, T1, B;
+  bool tiled;
+  float *xc, *z, *hp, *cs, *hs, *c0buf, *dhs, *dz, *dhrec, *dc0, *dc1, *dd;
+  unsigned int* counter;   // barrier counters of the tiled kernels
+};
+LstmCore lstm_core(int H, int CI, int T1, int B, bool tiled, const LstmBufs& o, void* ws, unsigned int* counter);
+// z = xc W + b; c0buf = c0; the recurrence -> z (activated gates), hs, cs, hp.
+int lstm_core_forward(const GemmRunner& g, const LstmCore& c, const float* W, const float* U, const float* b,
+                      const uint8_t* done, const float* h0, const float* c0, cudaStream_t st);
+// BPTT of dhs -> dz; dU = hp^T dz, dW = xc^T dz, db = column sums of dz; dd = (dz W[:H]^T) masked by
+// xc[:, :H] > 0 (the gradient of the ReLU'd Dense output at the head of the core input).
+int lstm_core_backward(const GemmRunner& g, const LstmCore& c, const float* W, const float* U,
+                       const uint8_t* done, float* dW, float* dU, float* db, cudaStream_t st);
 
 }  // namespace seedrl

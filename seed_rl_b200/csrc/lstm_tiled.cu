@@ -2,10 +2,10 @@
 // done-resets (dmlab/networks.py:157-169, atari/networks.py:176-218) -- forward and BPTT -- as ONE
 // launch each, CTA = (batch tile, unit group).
 //
-// The first form (lstm_persistent.cu: CTA = 2..4 hidden units, ALL batch rows) makes every one of its
-// 128 CTAs re-read the whole h[t] (64 KB) / dZ[t+1] (256 KB) through L2 each step and synchronises
-// all 128 CTAs with one grid barrier per step: 8.4 us (forward) / 18 us (backward) per step at
-// H = 256, B = 64.  Here a CTA owns NU = 16 hidden units x RB batch rows:
+// A CTA that owns a few hidden units for ALL batch rows (CTA = 2..4 units, 128 CTAs at H = 256) has to
+// re-read the whole h[t] (64 KB) / dZ[t+1] (256 KB) through L2 each step and synchronise all CTAs with
+// one grid barrier per step: measured at 8.4 us (forward) / 18 us (backward) per step at H = 256,
+// B = 64.  Here a CTA owns NU = 16 hidden units x RB batch rows:
 //   * it needs only ITS batch rows of h[t] / dZ[t+1] (8x less L2 traffic at B = 64),
 //   * it depends only on the CTAs of the SAME batch tile, so the per-step barrier is one counter per
 //     batch tile (H/16 arrivals) instead of one grid-wide counter -- batch tiles run independently,

@@ -8,8 +8,6 @@
 // (_baseline, _conv_to_linear, _core, _policy_logits, _stacks...), Keras layouts,
 // every tensor start aligned to 64 floats (256 B), then the scalar entropy_cost_param
 // (learner.py:225-234).
-#include <string.h>
-
 #include <vector>
 
 #include "kernels.h"
@@ -17,15 +15,6 @@
 namespace seedrl {
 
 constexpr int kHidden = 256;   // LSTMCell(256), Dense(256)
-constexpr size_t kAlignFloats = 64;
-
-struct ParamInfo {
-  std::string name;
-  int rank;
-  int64_t dims[4];
-  size_t offset;   // floats
-  size_t size;     // floats
-};
 
 struct ConvLayer {
   int cin, cout;
@@ -40,54 +29,28 @@ struct Stack {
 
 struct seedrl_net {
   seedrl_net_config cfg;
-  std::vector<seedrl::ParamInfo> params;   // network tensors, then entropy_cost_param
-  size_t arena_floats;
+  seedrl::ParamTable pt;                   // network tensors, then entropy_cost_param
   size_t logical_params;
   int p_base_w, p_base_b, p_dense_w, p_dense_b, p_core_w, p_core_u, p_core_b, p_pol_w, p_pol_b;
   std::vector<seedrl::Stack> stacks;       // deep
-  int sh_c0w, sh_c0b, sh_c1w, sh_c1b;      // shallow
-  int sh_h1, sh_w1, sh_h2, sh_w2;
+  seedrl::StridedConv sh[2];               // shallow: conv 8x8/4 -> 16, conv 4x4/2 -> 32
   int flat;                                // conv features fed to Dense(256)
-  int lstm_mode = 2;                       // 2 = tiled persistent kernels (lstm_tiled.cu), 1 = first persistent form, 0 = per-step launches
+  int lstm_mode = 2;                       // 2 = tiled persistent kernels (lstm_tiled.cu), 0 = per-step launches
   int conv_mode = 0;                       // 0 = fp32 SIMT, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3 (fp32-faithful)
   int core_in;                             // 256 + 1 + A
 };
 
 namespace seedrl {
 
-static int add_param(seedrl_net* n, const std::string& name, std::initializer_list<int64_t> dims) {
-  ParamInfo p;
-  p.name = name;
-  p.rank = (int)dims.size();
-  size_t sz = 1;
-  int i = 0;
-  for (int64_t d : dims) { p.dims[i++] = d; sz *= (size_t)d; }
-  for (; i < 4; ++i) p.dims[i] = 1;
-  p.size = sz;
-  p.offset = n->arena_floats;
-  n->arena_floats += (sz + kAlignFloats - 1) / kAlignFloats * kAlignFloats;
-  n->params.push_back(p);
-  return (int)n->params.size() - 1;
-}
-
 static ConvLayer add_conv(seedrl_net* n, const std::string& prefix, int k, int cin, int cout) {
   ConvLayer l;
   l.cin = cin; l.cout = cout;
-  l.w = add_param(n, prefix + "/kernel", {k, k, cin, cout});
-  l.b = add_param(n, prefix + "/bias", {cout});
+  l.w = n->pt.add(prefix + "/kernel", {k, k, cin, cout});
+  l.b = n->pt.add(prefix + "/bias", {cout});
   return l;
 }
 
 // ---- workspace plan -----------------------------------------------------------
-struct Bump {
-  size_t off = 0;
-  size_t take(size_t bytes) {
-    const size_t o = off;
-    off += (bytes + 255) / 256 * 256;
-    return o;
-  }
-};
-
 struct StackBufs {
   size_t a0, p, idx, c0, o0, c1, o1;
   // conv_mode 3 (plane tensors, conv_planes.cu): raw / ReLU'd pooled activation, ReLU'd c0 / c1,
@@ -105,9 +68,9 @@ struct Plan {
   std::vector<StackBufs> st;
   size_t sh_a1, sh_a2;         // shallow conv outputs (post-relu)
   size_t sh_col0, sh_col1;     // shallow net, tensor-core modes: im2col matrices (kept for the backward)
-  size_t xc, z, hp, cs, hs, c0buf;
+  LstmBufs lstm;
   // backward scratch
-  size_t dhs, dz, dhrec, dc0, dc1, dd, gA, gB, gC, gFull, wt, partial, wq, tcerr, counter, gemm_ws, wq_all, partial_all;
+  size_t gA, gB, gC, gFull, wt, partial, wq, tcerr, counter, gemm_ws, wq_all, partial_all;
   size_t gP1, gP2, gP3, gFP;   // conv_mode 3: plane-tensor gradients (pooled resolution x3, full resolution)
   size_t obs4, w0pad, dw0pad;  // 3-channel frames: zero-padded frames / first-conv weights / their gradient
   size_t total;
@@ -150,29 +113,20 @@ static Plan make_plan(const seedrl_net* n, int T1, int B) {
     }
     p.sh_a1 = p.sh_a2 = 0;
   } else {
-    const size_t a1 = N * n->sh_h1 * n->sh_w1 * 16, a2 = N * n->sh_h2 * n->sh_w2 * 32;
+    const StridedConv& c0 = n->sh[0];
+    const StridedConv& c1 = n->sh[1];
+    const size_t a1 = N * c0.hout * c0.wout * 16, a2 = N * c1.hout * c1.wout * 32;
     p.sh_a1 = b.take(a1 * 4);
     p.sh_a2 = b.take(a2 * 4);
     p.sh_col0 = p.sh_col1 = 0;
     if (n->conv_mode >= 1) {
-      p.sh_col0 = b.take(N * n->sh_h1 * n->sh_w1 * (size_t)(64 * n->cfg.obs_c) * 4);
-      p.sh_col1 = b.take(N * n->sh_h2 * n->sh_w2 * (size_t)(16 * 16) * 4);
+      p.sh_col0 = b.take(N * c0.hout * c0.wout * (size_t)(64 * n->cfg.obs_c) * 4);
+      p.sh_col1 = b.take(N * c1.hout * c1.wout * (size_t)(16 * 16) * 4);
     }
     pooled_max = a1 > a2 ? a1 : a2;
     full_max = 0;
   }
-  p.xc = b.take(N * n->core_in * 4);
-  p.z = b.take(N * 4 * kHidden * 4);
-  p.hp = b.take(N * kHidden * 4);
-  p.cs = b.take(N * kHidden * 4);
-  p.hs = b.take(N * kHidden * 4);
-  p.c0buf = b.take((size_t)B * kHidden * 4);
-  p.dhs = b.take(N * kHidden * 4);
-  p.dz = b.take(N * 4 * kHidden * 4);
-  p.dhrec = b.take((size_t)B * kHidden * 4);
-  p.dc0 = b.take((size_t)B * kHidden * 4);
-  p.dc1 = b.take((size_t)B * kHidden * 4);
-  p.dd = b.take(N * kHidden * 4);
+  p.lstm = lstm_bufs(&b, N, B, kHidden, n->core_in);
   p.obs4 = p.w0pad = p.dw0pad = 0;
   if (n->cfg.net == SEEDRL_NET_DEEP && n->cfg.obs_c == 3) {
     p.obs4 = b.take(N * n->cfg.obs_h * n->cfg.obs_w * 4);
@@ -203,11 +157,7 @@ static Plan make_plan(const seedrl_net* n, int T1, int B) {
   return p;
 }
 
-#define SEEDRL_TRY(expr)              \
-  do {                                \
-    const int rc__ = (expr);          \
-    if (rc__ != SEEDRL_OK) return rc__; \
-  } while (0)
+#define SEEDRL_TRY(expr) SEEDRL_TRY_RC(expr)
 
 // 3-channel frames (DMLab's 72x96x3, dmlab/env.py:44-54): the first convolution's kernels are built
 // for 4 input channels, so a forward/backward call works on a zero-padded copy of the frames and of
@@ -219,11 +169,11 @@ static thread_local const float* t_w0_pad = nullptr;
 static thread_local float* t_dw0_pad = nullptr;
 static inline const float* P(const seedrl_net* n, const float* arena, int idx) {
   if (idx == t_w0_index && t_w0_pad) return t_w0_pad;
-  return arena + n->params[idx].offset;
+  return n->pt.at(arena, idx);
 }
 static inline float* G(const seedrl_net* n, float* arena, int idx) {
   if (idx == t_w0_index && t_dw0_pad) return t_dw0_pad;
-  return arena + n->params[idx].offset;
+  return n->pt.at(arena, idx);
 }
 
 __global__ void pad_frames3_kernel(size_t npix, const uint8_t* __restrict__ src, uchar4* __restrict__ dst) {
@@ -244,20 +194,12 @@ __global__ void unpad_dw0_kernel(int cout, const float* __restrict__ dwp, float*
   const int co = i % cout, ci = (i / cout) % 3, tap = i / (3 * cout);
   dw[i] = dwp[(tap * 4 + ci) * cout + co];
 }
-template <typename T>
-static inline T* W(void* ws, size_t off) {
-  return reinterpret_cast<T*>(reinterpret_cast<char*>(ws) + off);
+// The dense contractions of the schedule run on the tensor cores in every tensor-core conv mode.
+static GemmRunner gemm_runner(const seedrl_net* n, void* ws, const Plan& pl) {
+  return GemmRunner{n->conv_mode >= 1, n->conv_mode >= 2, W<float>(ws, pl.gemm_ws), W<int>(ws, pl.tcerr)};
 }
-
-// One dense contraction of the schedule: tcgen05 when the net runs in tensor-core mode and the
-// shape is worth a 128-row tile, else the fp32 SIMT kernel.
-static int run_gemm(const seedrl_net* n, void* ws, const Plan& pl, bool ta, bool tb, int M, int N, int K,
-                    const float* A, int lda, const float* B, int ldb, float* C, int ldc, const GemmEpi& e,
-                    cudaStream_t st) {
-  if (n->conv_mode >= 1 && gemm_tc_supported(M, N, K))
-    return gemm_tc(ta, tb, n->conv_mode >= 2, M, N, K, A, lda, B, ldb, C, ldc, e, W<float>(ws, pl.gemm_ws),
-                   gemm_tc_workspace_bytes(), W<int>(ws, pl.tcerr), st);
-  return sgemm(ta, tb, M, N, K, A, lda, B, ldb, C, ldc, e, st);
+static LstmCore net_lstm_core(const seedrl_net* n, void* ws, const Plan& pl, int T1, int B) {
+  return lstm_core(kHidden, n->core_in, T1, B, n->lstm_mode == 2, pl.lstm, ws, W<unsigned int>(ws, pl.counter));
 }
 
 // Per-call context of the tensor-core path (thread-local: forward/backward of different nets
@@ -343,7 +285,7 @@ struct PadScope {
     pad_frames3_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, st>>>(npix, observation, W<uchar4>(ws, pl.obs4));
     count_launch(PC_MISC, st);
     const int wi = n->stacks[0].conv.w;
-    pad_w0_kernel<<<ceil_div(9 * 4 * 16, 128), 128, 0, st>>>(16, prm + n->params[wi].offset, W<float>(ws, pl.w0pad));
+    pad_w0_kernel<<<ceil_div(9 * 4 * 16, 128), 128, 0, st>>>(16, n->pt.at(prm, wi), W<float>(ws, pl.w0pad));
     count_launch(PC_MISC, st);
     if (cudaGetLastError() != cudaSuccess) rc = set_error(SEEDRL_ERR_INTERNAL, "3-channel padding launch failed");
     obs = W<uint8_t>(ws, pl.obs4);
@@ -362,12 +304,11 @@ extern "C" int seedrl_net_create(const seedrl_net_config* cfg, seedrl_net** out)
   SEEDRL_CHECK_ARG(cfg->num_actions >= 1 && cfg->obs_h > 0 && cfg->obs_w > 0, "bad shape");
   seedrl_net* n = new seedrl_net();
   n->cfg = *cfg;
-  n->arena_floats = 0;
   const int A = cfg->num_actions;
   n->core_in = kHidden + 1 + A;
   // tf.Module order: _baseline, _conv_to_linear, _core, _policy_logits, _stacks
-  n->p_base_w = add_param(n, "baseline/kernel", {kHidden, 1});
-  n->p_base_b = add_param(n, "baseline/bias", {1});
+  n->p_base_w = n->pt.add("baseline/kernel", {kHidden, 1});
+  n->p_base_b = n->pt.add("baseline/bias", {1});
   int flat = 0;
   if (cfg->net == SEEDRL_NET_DEEP) {
     if (cfg->obs_c != 4 && cfg->obs_c != 3) {
@@ -380,18 +321,18 @@ extern "C" int seedrl_net_create(const seedrl_net_config* cfg, seedrl_net** out)
     for (int s = 0; s < 3; ++s) { h = (h + 1) / 2; w = (w + 1) / 2; }
     flat = h * w * chans[2];
   } else {
-    n->sh_h1 = (cfg->obs_h - 8) / 4 + 1; n->sh_w1 = (cfg->obs_w - 8) / 4 + 1;
-    n->sh_h2 = (n->sh_h1 - 4) / 2 + 1;   n->sh_w2 = (n->sh_w1 - 4) / 2 + 1;
-    flat = n->sh_h2 * n->sh_w2 * 32;
+    n->sh[0] = strided_conv(8, 4, cfg->obs_c, 16, cfg->obs_h, cfg->obs_w);
+    n->sh[1] = strided_conv(4, 2, 16, 32, n->sh[0].hout, n->sh[0].wout);
+    flat = n->sh[1].hout * n->sh[1].wout * 32;
   }
   n->flat = flat;
-  n->p_dense_w = add_param(n, "conv_to_linear/kernel", {flat, kHidden});
-  n->p_dense_b = add_param(n, "conv_to_linear/bias", {kHidden});
-  n->p_core_w = add_param(n, "core/kernel", {n->core_in, 4 * kHidden});
-  n->p_core_u = add_param(n, "core/recurrent_kernel", {kHidden, 4 * kHidden});
-  n->p_core_b = add_param(n, "core/bias", {4 * kHidden});
-  n->p_pol_w = add_param(n, "policy_logits/kernel", {kHidden, A});
-  n->p_pol_b = add_param(n, "policy_logits/bias", {A});
+  n->p_dense_w = n->pt.add("conv_to_linear/kernel", {flat, kHidden});
+  n->p_dense_b = n->pt.add("conv_to_linear/bias", {kHidden});
+  n->p_core_w = n->pt.add("core/kernel", {n->core_in, 4 * kHidden});
+  n->p_core_u = n->pt.add("core/recurrent_kernel", {kHidden, 4 * kHidden});
+  n->p_core_b = n->pt.add("core/bias", {4 * kHidden});
+  n->p_pol_w = n->pt.add("policy_logits/kernel", {kHidden, A});
+  n->p_pol_b = n->pt.add("policy_logits/bias", {A});
   if (cfg->net == SEEDRL_NET_DEEP) {
     int h = cfg->obs_h, w = cfg->obs_w, c = cfg->obs_c;
     const int chans[3] = {16, 32, 32};
@@ -411,25 +352,27 @@ extern "C" int seedrl_net_create(const seedrl_net_config* cfg, seedrl_net** out)
       h = st.hout; w = st.wout; c = st.c;
     }
   } else {
-    ConvLayer c0 = add_conv(n, "conv0", 8, cfg->obs_c, 16);
-    ConvLayer c1 = add_conv(n, "conv1", 4, 16, 32);
-    n->sh_c0w = c0.w; n->sh_c0b = c0.b; n->sh_c1w = c1.w; n->sh_c1b = c1.b;
+    for (int i = 0; i < 2; ++i) {
+      const ConvLayer l = add_conv(n, "conv" + std::to_string(i), n->sh[i].k, n->sh[i].cin, n->sh[i].cout);
+      n->sh[i].w = l.w; n->sh[i].b = l.b;
+    }
   }
   n->logical_params = 0;
-  for (const ParamInfo& p : n->params) n->logical_params += p.size;
-  add_param(n, "entropy_cost_param", {});
+  for (const ParamInfo& p : n->pt.params) n->logical_params += p.size;
+  n->pt.add("entropy_cost_param", {});
   *out = n;
   return SEEDRL_OK;
 }
 
 extern "C" void seedrl_net_destroy(seedrl_net* net) { delete net; }
 extern "C" int seedrl_net_num_param_tensors(const seedrl_net* net) {
-  return net ? (int)net->params.size() - 1 : 0;
+  return net ? (int)net->pt.params.size() - 1 : 0;
 }
 extern "C" size_t seedrl_net_num_params(const seedrl_net* net) { return net ? net->logical_params : 0; }
-extern "C" size_t seedrl_net_arena_floats(const seedrl_net* net) { return net ? net->arena_floats : 0; }
+extern "C" size_t seedrl_net_arena_floats(const seedrl_net* net) { return net ? net->pt.arena_floats : 0; }
 extern "C" int seedrl_net_set_lstm_mode(seedrl_net* net, int mode) {
-  SEEDRL_CHECK_ARG(net && mode >= 0 && mode <= 2, "mode must be 0 (per-step launches), 1 (persistent, CTA = 2 units) or 2 (persistent, CTA = batch tile x 16 units)");
+  SEEDRL_CHECK_ARG(net && (mode == 0 || mode == 2),
+                   "mode must be 0 (per-step launches) or 2 (persistent, CTA = batch tile x 16 units)");
   net->lstm_mode = mode;
   return SEEDRL_OK;
 }
@@ -443,15 +386,7 @@ extern "C" int seedrl_net_set_conv_mode(seedrl_net* net, int mode) {
 
 extern "C" int seedrl_net_param_info(const seedrl_net* net, int index, char* name_buf,
                                      size_t name_buf_len, int64_t* dims, size_t* offset) {
-  if (!net || index < 0 || index >= (int)net->params.size()) return -1;
-  const ParamInfo& p = net->params[index];
-  if (name_buf && name_buf_len) {
-    strncpy(name_buf, p.name.c_str(), name_buf_len - 1);
-    name_buf[name_buf_len - 1] = 0;
-  }
-  if (dims) for (int i = 0; i < 4; ++i) dims[i] = p.dims[i];
-  if (offset) *offset = p.offset;
-  return p.rank;
+  return net ? net->pt.info(index, name_buf, name_buf_len, dims, offset) : -1;
 }
 
 extern "C" size_t seedrl_net_workspace_bytes(const seedrl_net* net, int T1, int B) {
@@ -550,55 +485,25 @@ static int torso_forward_planes(const seedrl_net* n, const float* prm, const Pla
   return SEEDRL_OK;
 }
 
-// Shallow net, tensor-core modes: layer 0 = conv 8x8/4 on the uint8 frames, layer 1 = conv 4x4/2 on a1.
-static bool shallow_gathered(const seedrl_net* n, int layer, int N, const void* x, ConvGather* cg) {
-  if (n->conv_mode < 1 || !gemm_tc_gather_enabled()) return false;
-  if (layer == 0)
-    return gemm_tc_supported(N * n->sh_h1 * n->sh_w1, 16, 64 * n->cfg.obs_c) &&
-           conv_gather_setup(x, 1, N, n->cfg.obs_h, n->cfg.obs_w, n->cfg.obs_c, 8, 4, cg);
-  return gemm_tc_supported(N * n->sh_h2 * n->sh_w2, 32, 256) && conv_gather_setup(x, 0, N, n->sh_h1, n->sh_w1, 16, 4, 2, cg);
-}
-static int run_gemm_gather(const seedrl_net* n, void* ws, const Plan& pl, bool ta, int M, int N, int K,
-                           const ConvGather& cg, const float* B, int ldb, float* C, int ldc, const GemmEpi& e,
-                           cudaStream_t st) {
-  return gemm_tc(ta, false, n->conv_mode >= 2, M, N, K, nullptr, 0, B, ldb, C, ldc, e, W<float>(ws, pl.gemm_ws),
-                 gemm_tc_workspace_bytes(), W<int>(ws, pl.tcerr), st, &cg);
-}
-
+// Shallow net: layer 0 = conv 8x8/4 on the uint8 frames, layer 1 = conv 4x4/2 on a1.
 static int torso_forward_shallow(const seedrl_net* n, const float* prm, const Plan& pl,
                                  const uint8_t* obs, void* ws, cudaStream_t st) {
   const int N = pl.N;
+  const StridedConv& c0 = n->sh[0];
+  const StridedConv& c1 = n->sh[1];
   float* a1 = W<float>(ws, pl.sh_a1);
   float* a2 = W<float>(ws, pl.sh_a2);
   if (n->conv_mode >= 1 && n->cfg.obs_c % 4 == 0) {
-    // tensor-core modes: im2col + tcgen05 GEMM with bias + ReLU in the epilogue (the R2D2 body's path)
-    const int C = n->cfg.obs_c, K0 = 64 * C, K1 = 16 * 16;
-    float* col0 = W<float>(ws, pl.sh_col0); float* col1 = W<float>(ws, pl.sh_col1);
-    GemmEpi e = epi_none();
-    e.bias = P(n, prm, n->sh_c0b); e.relu = 1;
-    const int M0 = N * n->sh_h1 * n->sh_w1, M1 = N * n->sh_h2 * n->sh_w2;
-    // the im2col matrices are gathered inside the GEMM's operand staging where the geometry allows it
-    // (kernels.h ConvGather); otherwise materialised (and kept for the weight gradient)
-    ConvGather cg;
-    if (shallow_gathered(n, 0, N, obs, &cg)) {
-      SEEDRL_TRY(run_gemm_gather(n, ws, pl, false, M0, 16, K0, cg, P(n, prm, n->sh_c0w), 16, a1, 16, e, st));
-    } else {
-      SEEDRL_TRY(im2col_nhwc(N, n->cfg.obs_h, n->cfg.obs_w, C, 8, 4, 1, obs, col0, st));
-      SEEDRL_TRY(run_gemm(n, ws, pl, false, false, M0, 16, K0, col0, K0, P(n, prm, n->sh_c0w), 16, a1, 16, e, st));
-    }
-    e.bias = P(n, prm, n->sh_c1b);
-    if (shallow_gathered(n, 1, N, a1, &cg)) {
-      SEEDRL_TRY(run_gemm_gather(n, ws, pl, false, M1, 32, K1, cg, P(n, prm, n->sh_c1w), 32, a2, 32, e, st));
-    } else {
-      SEEDRL_TRY(im2col_nhwc(N, n->sh_h1, n->sh_w1, 16, 4, 2, 0, a1, col1, st));
-      SEEDRL_TRY(run_gemm(n, ws, pl, false, false, M1, 32, K1, col1, K1, P(n, prm, n->sh_c1w), 32, a2, 32, e, st));
-    }
-    return SEEDRL_OK;
+    // tensor-core modes: GEMMs over the im2col matrices, bias + ReLU in the epilogue (as the R2D2 body)
+    const GemmRunner g = gemm_runner(n, ws, pl);
+    SEEDRL_TRY(strided_conv_forward(g, N, c0, true, obs, P(n, prm, c0.w), P(n, prm, c0.b), W<float>(ws, pl.sh_col0),
+                                    a1, st));
+    return strided_conv_forward(g, N, c1, false, a1, P(n, prm, c1.w), P(n, prm, c1.b), W<float>(ws, pl.sh_col1), a2,
+                                st);
   }
-  SEEDRL_TRY(convgen_forward(N, n->cfg.obs_h, n->cfg.obs_w, n->cfg.obs_c, 16, 8, 4, 1, obs,
-                             P(n, prm, n->sh_c0w), P(n, prm, n->sh_c0b), 1, a1, st));
-  SEEDRL_TRY(convgen_forward(N, n->sh_h1, n->sh_w1, 16, 32, 4, 2, 0, a1, P(n, prm, n->sh_c1w),
-                             P(n, prm, n->sh_c1b), 1, a2, st));
+  SEEDRL_TRY(convgen_forward(N, c0.hin, c0.win, c0.cin, 16, 8, 4, 1, obs, P(n, prm, c0.w), P(n, prm, c0.b), 1, a1,
+                             st));
+  SEEDRL_TRY(convgen_forward(N, c1.hin, c1.win, 16, 32, 4, 2, 0, a1, P(n, prm, c1.w), P(n, prm, c1.b), 1, a2, st));
   return SEEDRL_OK;
 }
 
@@ -639,55 +544,25 @@ extern "C" int seedrl_net_forward(const seedrl_net* n, const float* prm, int T1,
     flat_src = W<float>(ws, pl.sh_a2);
     flat_relu = 0;                         // already relu'd
   }
-  float* xc = W<float>(ws, pl.xc);
-  float* z = W<float>(ws, pl.z);
-  float* hp = W<float>(ws, pl.hp);
-  float* cs = W<float>(ws, pl.cs);
-  float* hs = W<float>(ws, pl.hs);
-  float* c0buf = W<float>(ws, pl.c0buf);
+  const GemmRunner g = gemm_runner(n, ws, pl);
+  const LstmCore core = net_lstm_core(n, ws, pl, T1, B);
+  float* xc = core.xc;
+  float* hs = core.hs;
+  float* cs = core.cs;
   // Dense(256) + relu written straight into the first 256 columns of the core input
   GemmEpi e = epi_none();
   e.bias = P(n, prm, n->p_dense_b); e.relu = 1; e.a_relu = flat_relu;
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, false, N, kHidden, n->flat, flat_src, n->flat, P(n, prm, n->p_dense_w),
-                   kHidden, xc, CI, e, st));
+  SEEDRL_TRY(g.gemm(false, false, N, kHidden, n->flat, flat_src, n->flat, P(n, prm, n->p_dense_w), kHidden, xc, CI,
+                    e, st));
   SEEDRL_TRY(core_input_tail(N, kHidden, A, reward, prev_actions, xc, st));
-  // input projection for all T at once: z = xc W + b
-  e = epi_none();
-  e.bias = P(n, prm, n->p_core_b);
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, false, N, 4 * kHidden, CI, xc, CI, P(n, prm, n->p_core_w), 4 * kHidden, z,
-                   4 * kHidden, e, st));
-  SEEDRL_CUDA(cudaMemcpyAsync(c0buf, c0, (size_t)B * kHidden * 4, cudaMemcpyDeviceToDevice, st));
-  GemmEpi eacc = epi_none();
-  eacc.accumulate = 1;
-  if (n->lstm_mode == 2) {
-    // one kernel for the whole recurrence, CTA = (batch tile, 16 units) (lstm_tiled.cu)
-    SEEDRL_TRY(lstm_forward_tiled(kHidden, T1, B, P(n, prm, n->p_core_u), done, z, h0, c0buf, hs, cs, hp,
-                                  W<unsigned int>(ws, pl.counter), W<int>(ws, pl.tcerr), st));
-  } else if (n->lstm_mode == 1) {
-    // one cooperative kernel for the whole recurrence (lstm_persistent.cu)
-    SEEDRL_TRY(lstm_forward_persistent(kHidden, T1, B, P(n, prm, n->p_core_u), done, z, h0, c0buf, hs, cs, hp,
-                                       W<unsigned int>(ws, pl.counter), W<int>(ws, pl.tcerr), st));
-  } else {
-    SEEDRL_TRY(lstm_mask_state(B, kHidden, done, h0, hp, st));
-  }
-  for (int t = 0; t < T1 && n->lstm_mode == 0; ++t) {
-    float* zt = z + (size_t)t * B * 4 * kHidden;
-    SEEDRL_TRY(run_gemm(n, ws, pl, false, false, B, 4 * kHidden, kHidden, hp + (size_t)t * B * kHidden, kHidden,
-                     P(n, prm, n->p_core_u), 4 * kHidden, zt, 4 * kHidden, eacc, st));
-    const bool last = (t + 1 == T1);
-    SEEDRL_TRY(lstm_pointwise_fwd(B, kHidden, zt, t == 0 ? c0buf : cs + (size_t)(t - 1) * B * kHidden,
-                                  done + (size_t)t * B, last ? nullptr : done + (size_t)(t + 1) * B,
-                                  cs + (size_t)t * B * kHidden, hs + (size_t)t * B * kHidden,
-                                  last ? nullptr : hp + (size_t)(t + 1) * B * kHidden, st));
-  }
+  SEEDRL_TRY(lstm_core_forward(g, core, P(n, prm, n->p_core_w), P(n, prm, n->p_core_u), P(n, prm, n->p_core_b), done,
+                               h0, c0, st));
   // heads, networks.py:116-118
   e = epi_none();
   e.bias = P(n, prm, n->p_pol_b);
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, false, N, A, kHidden, hs, kHidden, P(n, prm, n->p_pol_w), A, policy_logits,
-                   A, e, st));
+  SEEDRL_TRY(g.gemm(false, false, N, A, kHidden, hs, kHidden, P(n, prm, n->p_pol_w), A, policy_logits, A, e, st));
   e.bias = P(n, prm, n->p_base_b);
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, false, N, 1, kHidden, hs, kHidden, P(n, prm, n->p_base_w), 1, baseline, 1,
-                   e, st));
+  SEEDRL_TRY(g.gemm(false, false, N, 1, kHidden, hs, kHidden, P(n, prm, n->p_base_w), 1, baseline, 1, e, st));
   if (h_out)
     SEEDRL_CUDA(cudaMemcpyAsync(h_out, hs + (size_t)(T1 - 1) * B * kHidden, (size_t)B * kHidden * 4,
                                 cudaMemcpyDeviceToDevice, st));
@@ -705,14 +580,7 @@ extern "C" int seedrl_net_check_error(const seedrl_net* n, int T1, int B, void* 
   SEEDRL_CHECK_ARG(n && ws && T1 >= 1 && B >= 1, "bad arguments");
   const Plan pl = make_plan(n, T1, B);
   SEEDRL_CHECK_ARG(ws_bytes >= pl.total, "workspace too small");
-  int flag = 0;
-  SEEDRL_CUDA(cudaMemcpyAsync(&flag, W<int>(ws, pl.tcerr), sizeof(int), cudaMemcpyDeviceToHost,
-                              (cudaStream_t)stream));
-  SEEDRL_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-  if (flag != 0)
-    return set_error(SEEDRL_ERR_INTERNAL,
-                     "a tensor-core / persistent kernel timed out on a barrier: results of this step are invalid");
-  return SEEDRL_OK;
+  return read_error_flag(W<int>(ws, pl.tcerr), (cudaStream_t)stream);
 }
 
 // ---- backward -------------------------------------------------------------------
@@ -827,35 +695,22 @@ static int torso_backward_shallow(const seedrl_net* n, const float* prm, float* 
                                   const uint8_t* obs, void* ws, cudaStream_t st) {
   // On entry gA holds d loss / d a2 (already masked by a2 > 0).
   const int N = pl.N;
+  const StridedConv& c0 = n->sh[0];
+  const StridedConv& c1 = n->sh[1];
   float* gA = W<float>(ws, pl.gA); float* gB = W<float>(ws, pl.gB);
   const float* a1 = W<float>(ws, pl.sh_a1);
   if (n->conv_mode >= 1 && n->cfg.obs_c % 4 == 0) {
-    const int C = n->cfg.obs_c, K0 = 64 * C, K1 = 16 * 16;
-    const int M1 = N * n->sh_h2 * n->sh_w2, M0 = N * n->sh_h1 * n->sh_w1;
-    float* col0 = W<float>(ws, pl.sh_col0); float* col1 = W<float>(ws, pl.sh_col1);
-    const GemmEpi e0 = epi_none();
-    ConvGather cg;
-    if (shallow_gathered(n, 1, N, a1, &cg))
-      SEEDRL_TRY(run_gemm_gather(n, ws, pl, true, K1, 32, M1, cg, gA, 32, G(n, grd, n->sh_c1w), 32, e0, st));
-    else
-      SEEDRL_TRY(run_gemm(n, ws, pl, true, false, K1, 32, M1, col1, K1, gA, 32, G(n, grd, n->sh_c1w), 32, e0, st));
-    SEEDRL_TRY(colsum(M1, 32, gA, 32, G(n, grd, n->sh_c1b), st, W<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-    SEEDRL_TRY(run_gemm(n, ws, pl, false, true, M1, K1, 32, gA, 32, P(n, prm, n->sh_c1w), 32, col1, K1, e0, st));
-    SEEDRL_TRY(col2im_nhwc(N, n->sh_h1, n->sh_w1, 16, 4, 2, col1, a1, gB, st));
-    if (shallow_gathered(n, 0, N, obs, &cg))
-      SEEDRL_TRY(run_gemm_gather(n, ws, pl, true, K0, 16, M0, cg, gB, 16, G(n, grd, n->sh_c0w), 16, e0, st));
-    else
-      SEEDRL_TRY(run_gemm(n, ws, pl, true, false, K0, 16, M0, col0, K0, gB, 16, G(n, grd, n->sh_c0w), 16, e0, st));
-    SEEDRL_TRY(colsum(M0, 16, gB, 16, G(n, grd, n->sh_c0b), st, W<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-    return SEEDRL_OK;
+    const GemmRunner g = gemm_runner(n, ws, pl);
+    SEEDRL_TRY(strided_conv_backward(g, N, c1, false, a1, W<float>(ws, pl.sh_col1), P(n, prm, c1.w), gA,
+                                     G(n, grd, c1.w), G(n, grd, c1.b), gB, st));
+    return strided_conv_backward(g, N, c0, true, obs, W<float>(ws, pl.sh_col0), P(n, prm, c0.w), gB, G(n, grd, c0.w),
+                                 G(n, grd, c0.b), nullptr, st);
   }
-  SEEDRL_TRY(convgen_wgrad(N, n->sh_h1, n->sh_w1, 16, 32, 4, 2, 0, a1, gA, G(n, grd, n->sh_c1w),
-                           G(n, grd, n->sh_c1b), W<float>(ws, pl.partial),
-                           conv3x3_wgrad_partial_bytes(), st));
-  SEEDRL_TRY(convgen_dgrad(N, n->sh_h1, n->sh_w1, 16, 32, 4, 2, gA, P(n, prm, n->sh_c1w), a1, gB, st));
-  SEEDRL_TRY(convgen_wgrad(N, n->cfg.obs_h, n->cfg.obs_w, n->cfg.obs_c, 16, 8, 4, 1, obs, gB,
-                           G(n, grd, n->sh_c0w), G(n, grd, n->sh_c0b), W<float>(ws, pl.partial),
-                           conv3x3_wgrad_partial_bytes(), st));
+  SEEDRL_TRY(convgen_wgrad(N, c1.hin, c1.win, 16, 32, 4, 2, 0, a1, gA, G(n, grd, c1.w), G(n, grd, c1.b),
+                           W<float>(ws, pl.partial), conv3x3_wgrad_partial_bytes(), st));
+  SEEDRL_TRY(convgen_dgrad(N, c1.hin, c1.win, 16, 32, 4, 2, gA, P(n, prm, c1.w), a1, gB, st));
+  SEEDRL_TRY(convgen_wgrad(N, c0.hin, c0.win, c0.cin, 16, 8, 4, 1, obs, gB, G(n, grd, c0.w), G(n, grd, c0.b),
+                           W<float>(ws, pl.partial), conv3x3_wgrad_partial_bytes(), st));
   return SEEDRL_OK;
 }
 
@@ -870,71 +725,42 @@ extern "C" int seedrl_net_backward(const seedrl_net* n, const float* prm, int T1
   const Plan pl = make_plan(n, T1, B);
   SEEDRL_CHECK_ARG(ws_bytes >= pl.total, "workspace too small");
   cudaStream_t st = (cudaStream_t)stream;
-  const int N = pl.N, A = n->cfg.num_actions, CI = n->core_in;
-  float* xc = W<float>(ws, pl.xc); float* z = W<float>(ws, pl.z);
-  float* hp = W<float>(ws, pl.hp); float* cs = W<float>(ws, pl.cs);
-  float* hs = W<float>(ws, pl.hs); float* c0buf = W<float>(ws, pl.c0buf);
-  float* dhs = W<float>(ws, pl.dhs); float* dz = W<float>(ws, pl.dz);
-  float* dhrec = W<float>(ws, pl.dhrec); float* dd = W<float>(ws, pl.dd);
-  float* dcb[2] = {W<float>(ws, pl.dc0), W<float>(ws, pl.dc1)};
+  const int N = pl.N, A = n->cfg.num_actions;
+  const GemmRunner g = gemm_runner(n, ws, pl);
+  const LstmCore core = net_lstm_core(n, ws, pl, T1, B);
+  float* hs = core.hs;
+  float* dhs = core.dhs;
+  float* dd = core.dd;
   // padding floats and the entropy_cost_param slot must not carry garbage into Adam / all-reduce
-  SEEDRL_CUDA(cudaMemsetAsync(grd, 0, n->arena_floats * sizeof(float), st));
+  SEEDRL_CUDA(cudaMemsetAsync(grd, 0, n->pt.arena_floats * sizeof(float), st));
 
   // heads
   GemmEpi e = epi_none();
-  SEEDRL_TRY(run_gemm(n, ws, pl, true, false, kHidden, A, N, hs, kHidden, dlogits, A, G(n, grd, n->p_pol_w), A, e, st));
-  SEEDRL_TRY(colsum(N, A, dlogits, A, G(n, grd, n->p_pol_b), st, W<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-  SEEDRL_TRY(run_gemm(n, ws, pl, true, false, kHidden, 1, N, hs, kHidden, dbaseline, 1, G(n, grd, n->p_base_w), 1, e, st));
-  SEEDRL_TRY(colsum(N, 1, dbaseline, 1, G(n, grd, n->p_base_b), st, W<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, true, N, kHidden, A, dlogits, A, P(n, prm, n->p_pol_w), A, dhs, kHidden, e, st));
+  SEEDRL_TRY(g.gemm(true, false, kHidden, A, N, hs, kHidden, dlogits, A, G(n, grd, n->p_pol_w), A, e, st));
+  SEEDRL_TRY(g.colsum(N, A, dlogits, A, G(n, grd, n->p_pol_b), st));
+  SEEDRL_TRY(g.gemm(true, false, kHidden, 1, N, hs, kHidden, dbaseline, 1, G(n, grd, n->p_base_w), 1, e, st));
+  SEEDRL_TRY(g.colsum(N, 1, dbaseline, 1, G(n, grd, n->p_base_b), st));
+  SEEDRL_TRY(g.gemm(false, true, N, kHidden, A, dlogits, A, P(n, prm, n->p_pol_w), A, dhs, kHidden, e, st));
   GemmEpi eacc = epi_none();
   eacc.accumulate = 1;
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, true, N, kHidden, 1, dbaseline, 1, P(n, prm, n->p_base_w), 1, dhs, kHidden,
-                   eacc, st));
-  // BPTT
-  if (n->lstm_mode == 2)
-    SEEDRL_TRY(lstm_backward_tiled(kHidden, T1, B, P(n, prm, n->p_core_u), done, z, cs, c0buf, dhs, dz,
-                                   W<unsigned int>(ws, pl.counter), W<int>(ws, pl.tcerr), st));
-  if (n->lstm_mode == 1)
-    SEEDRL_TRY(lstm_backward_persistent(kHidden, T1, B, P(n, prm, n->p_core_u), done, z, cs, c0buf, dhs, dz,
-                                        W<unsigned int>(ws, pl.counter), W<int>(ws, pl.tcerr), st));
-  for (int t = T1 - 1; t >= 0 && n->lstm_mode == 0; --t) {
-    const bool last = (t + 1 == T1);
-    const size_t o = (size_t)t * B * kHidden;
-    SEEDRL_TRY(lstm_pointwise_bwd(B, kHidden, z + (size_t)t * B * 4 * kHidden, cs + o,
-                                  t == 0 ? c0buf : cs + o - (size_t)B * kHidden, done + (size_t)t * B,
-                                  last ? nullptr : done + (size_t)(t + 1) * B, dhs + o,
-                                  last ? nullptr : dhrec, last ? nullptr : dcb[(t + 1) & 1],
-                                  dz + (size_t)t * B * 4 * kHidden, dcb[t & 1], st));
-    if (t > 0)
-      SEEDRL_TRY(run_gemm(n, ws, pl, false, true, B, kHidden, 4 * kHidden, dz + (size_t)t * B * 4 * kHidden,
-                       4 * kHidden, P(n, prm, n->p_core_u), 4 * kHidden, dhrec, kHidden, e, st));
-  }
-  SEEDRL_TRY(run_gemm(n, ws, pl, true, false, kHidden, 4 * kHidden, N, hp, kHidden, dz, 4 * kHidden,
-                   G(n, grd, n->p_core_u), 4 * kHidden, e, st));
-  SEEDRL_TRY(run_gemm(n, ws, pl, true, false, CI, 4 * kHidden, N, xc, CI, dz, 4 * kHidden, G(n, grd, n->p_core_w),
-                   4 * kHidden, e, st));
-  SEEDRL_TRY(colsum(N, 4 * kHidden, dz, 4 * kHidden, G(n, grd, n->p_core_b), st, W<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-  // d dense_out = (dz W[:256,:]^T) * (dense_out > 0)
-  GemmEpi em = epi_none();
-  em.mask = xc; em.ldm = CI;
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, true, N, kHidden, 4 * kHidden, dz, 4 * kHidden, P(n, prm, n->p_core_w),
-                   4 * kHidden, dd, kHidden, em, st));
+  SEEDRL_TRY(g.gemm(false, true, N, kHidden, 1, dbaseline, 1, P(n, prm, n->p_base_w), 1, dhs, kHidden, eacc, st));
+  SEEDRL_TRY(lstm_core_backward(g, core, P(n, prm, n->p_core_w), P(n, prm, n->p_core_u), done, G(n, grd, n->p_core_w),
+                                G(n, grd, n->p_core_u), G(n, grd, n->p_core_b), st));
   // Dense(256)
   const float* flat_src = n->cfg.net == SEEDRL_NET_DEEP ? W<float>(ws, pl.st.back().o1)
                                                         : W<float>(ws, pl.sh_a2);
   GemmEpi ea = epi_none();
   ea.a_relu = n->cfg.net == SEEDRL_NET_DEEP ? 1 : 0;
-  SEEDRL_TRY(run_gemm(n, ws, pl, true, false, n->flat, kHidden, N, flat_src, n->flat, dd, kHidden,
-                   G(n, grd, n->p_dense_w), kHidden, ea, st));
-  SEEDRL_TRY(colsum(N, kHidden, dd, kHidden, G(n, grd, n->p_dense_b), st, W<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
+  SEEDRL_TRY(g.gemm(true, false, n->flat, kHidden, N, flat_src, n->flat, dd, kHidden, G(n, grd, n->p_dense_w), kHidden,
+                    ea, st));
+  SEEDRL_TRY(g.colsum(N, kHidden, dd, kHidden, G(n, grd, n->p_dense_b), st));
   // every gradient of the arena's first bucket (heads, Dense, LSTM: floats [0, seedrl_net_grad_split))
   // is final here -- the conv torso's backward below only writes the second bucket
   if (t_head_ready) SEEDRL_CUDA(cudaEventRecord((cudaEvent_t)t_head_ready, st));
   GemmEpi ef = epi_none();
   ef.mask = flat_src; ef.ldm = n->flat;
-  SEEDRL_TRY(run_gemm(n, ws, pl, false, true, N, n->flat, kHidden, dd, kHidden, P(n, prm, n->p_dense_w), kHidden,
-                   W<float>(ws, pl.gA), n->flat, ef, st));
+  SEEDRL_TRY(g.gemm(false, true, N, n->flat, kHidden, dd, kHidden, P(n, prm, n->p_dense_w), kHidden,
+                    W<float>(ws, pl.gA), n->flat, ef, st));
   if (n->cfg.net == SEEDRL_NET_DEEP) {
     StepCtx ctx;
     ctx.wb = WgradBatch{W<float>(ws, pl.partial_all), kPartialAllBytes / sizeof(float), 0, 0, {}};
@@ -949,7 +775,7 @@ extern "C" int seedrl_net_backward(const seedrl_net* n, const float* prm, int T1
     if (rc_t == SEEDRL_OK) rc_t = wgrad_reduce_batch(&ctx.wb, st);
     if (rc_t == SEEDRL_OK && pad.active) {        // padded [3,3,4,16] gradient -> the [3,3,3,16] parameter slot
       unpad_dw0_kernel<<<ceil_div(9 * 3 * 16, 128), 128, 0, st>>>(16, W<float>(ws, pl.dw0pad),
-                                                                   grd + n->params[n->stacks[0].conv.w].offset);
+                                                                   n->pt.at(grd, n->stacks[0].conv.w));
       count_launch(PC_MISC, st);
     }
     return rc_t;
@@ -976,8 +802,8 @@ extern "C" int seedrl_net_backward_overlap(const seedrl_net* n, const float* prm
 }
 extern "C" size_t seedrl_net_grad_split(const seedrl_net* n) {
   if (!n) return 0;
-  const int first_conv = n->cfg.net == SEEDRL_NET_DEEP ? n->stacks[0].conv.w : n->sh_c0w;
-  return n->params[first_conv].offset;
+  const int first_conv = n->cfg.net == SEEDRL_NET_DEEP ? n->stacks[0].conv.w : n->sh[0].w;
+  return n->pt.params[first_conv].offset;
 }
 
 // ---- single-kernel test hooks (exported so the GPU parity tests can localise a

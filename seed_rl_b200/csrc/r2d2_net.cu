@@ -4,7 +4,8 @@
 // backward (what tf.GradientTape computes at agents/r2d2/learner.py:596-609).
 //
 // The three 'valid' strided convolutions (8x8/4 -> 32, 4x4/2 -> 64, 3x3/1 -> 64) run as
-// im2col + tensor-core GEMM (gemm_tc_kernel, bf16x3 = fp32-faithful; fp32 SIMT sgemm in mode 0):
+// im2col + tensor-core GEMM (net_common.cu strided_conv_*; gemm_tc_kernel, bf16x3 = fp32-faithful;
+// fp32 SIMT sgemm in mode 0):
 //   forward   col = im2col(x);  y = relu(col W + b)           (W is Keras HWIO = [k*k*cin, cout])
 //   weights   dW = col^T dy (deterministic split-K), db = column sums of dy
 //   data      dcol = dy W^T (written over col), dx = col2im(dcol) * (x > 0)   (gather form, no atomics)
@@ -14,10 +15,6 @@
 //
 // Parameters: one flat fp32 arena in tf.Module.trainable_variables order (attribute-name order:
 // _advantage, _body, _core, _value), Keras layouts, tensor starts aligned to 64 floats.
-#include <string.h>
-
-#include <vector>
-
 #include "kernels.h"
 
 #define SEEDRL_TRY(expr) SEEDRL_TRY_RC(expr)
@@ -25,81 +22,43 @@
 namespace seedrl {
 
 constexpr int kRH = 512;                 // LSTMCell(512), Dense(512) (networks.py:240-252)
-constexpr size_t kRAlign = 64;
-
-struct RParam {
-  std::string name;
-  int rank;
-  int64_t dims[4];
-  size_t offset, size;
-};
-struct RConv { int k, s, cin, cout, hin, win, hout, wout, w, b; };
 
 }  // namespace seedrl
 
 struct seedrl_r2d2_net {
   int A, H, W, C;
   int mode;                               // 0 = fp32 SIMT GEMMs, 2 = tcgen05 bf16x3
-  int lstm_mode = 2;                      // 2 = tiled persistent LSTM (lstm_tiled.cu), 1 = first persistent form
-  std::vector<seedrl::RParam> params;
-  size_t arena_floats, logical_params;
-  seedrl::RConv conv[3];
+  int lstm_mode = 2;                      // 2 = tiled persistent LSTM (lstm_tiled.cu), 0 = per-step launches
+  seedrl::ParamTable pt;
+  size_t logical_params;
+  seedrl::StridedConv conv[3];
   int flat, core_in;
   int p_ah_w, p_ah_b, p_a_w, p_dense_w, p_dense_b, p_core_w, p_core_u, p_core_b, p_vh_w, p_vh_b, p_v_w, p_v_b;
 };
 
 namespace seedrl {
 
-static int r_add(seedrl_r2d2_net* n, const std::string& name, std::initializer_list<int64_t> dims) {
-  RParam p;
-  p.name = name;
-  p.rank = (int)dims.size();
-  size_t sz = 1;
-  int i = 0;
-  for (int64_t d : dims) { p.dims[i++] = d; sz *= (size_t)d; }
-  for (; i < 4; ++i) p.dims[i] = 1;
-  p.size = sz;
-  p.offset = n->arena_floats;
-  n->arena_floats += (sz + kRAlign - 1) / kRAlign * kRAlign;
-  n->params.push_back(p);
-  return (int)n->params.size() - 1;
-}
-
-struct RBump {
-  size_t off = 0;
-  size_t take(size_t bytes) {
-    const size_t o = off;
-    off += (bytes + 255) / 256 * 256;
-    return o;
-  }
-};
-
 struct RPlan {
   size_t N;
   size_t col[3], act[3];                  // im2col matrices, post-ReLU conv outputs (NHWC)
-  size_t xc, z, hp, cs, hs, c0buf, vh, ah, v, adv;
-  size_t dv, dadv, dvh, dah, dhs, dz, dd, g[3];
+  LstmBufs lstm;
+  size_t vh, ah, v, adv, dv, dadv, dvh, dah, g[3];
   size_t gemm_ws, tcerr, counter;
   size_t total;
 };
 
 static RPlan r_plan(const seedrl_r2d2_net* n, int T, int B) {
   RPlan p;
-  RBump b;
+  Bump b;
   const size_t N = (size_t)T * B;
   p.N = N;
   for (int i = 0; i < 3; ++i) {
-    const RConv& c = n->conv[i];
+    const StridedConv& c = n->conv[i];
     p.col[i] = b.take(N * c.hout * c.wout * (size_t)(c.k * c.k * c.cin) * 4);
     p.act[i] = b.take(N * c.hout * c.wout * (size_t)c.cout * 4);
     p.g[i] = b.take(N * c.hout * c.wout * (size_t)c.cout * 4);
   }
-  p.xc = b.take(N * (size_t)n->core_in * 4);
-  p.z = b.take(N * 4 * kRH * 4);
-  p.hp = b.take(N * kRH * 4);
-  p.cs = b.take(N * kRH * 4);
-  p.hs = b.take(N * kRH * 4);
-  p.c0buf = b.take((size_t)B * kRH * 4);
+  p.lstm = lstm_bufs(&b, N, B, kRH, n->core_in);
   p.vh = b.take(N * kRH * 4);
   p.ah = b.take(N * kRH * 4);
   p.v = b.take(N * 4);
@@ -108,9 +67,6 @@ static RPlan r_plan(const seedrl_r2d2_net* n, int T, int B) {
   p.dadv = b.take(N * (size_t)n->A * 4);
   p.dvh = b.take(N * kRH * 4);
   p.dah = b.take(N * kRH * 4);
-  p.dhs = b.take(N * kRH * 4);
-  p.dz = b.take(N * 4 * kRH * 4);
-  p.dd = b.take(N * kRH * 4);
   p.gemm_ws = b.take(gemm_tc_workspace_bytes());
   p.tcerr = b.take(256);
   p.counter = b.take(256);
@@ -118,148 +74,12 @@ static RPlan r_plan(const seedrl_r2d2_net* n, int T, int B) {
   return p;
 }
 
-static int im2col(int N, const RConv& c, bool u8, const void* x, float* col, cudaStream_t st);
-static int col2im(int N, const RConv& c, const float* dcol, const float* xmask, float* dx, cudaStream_t st);
-
-template <typename T>
-static inline T* RW(void* ws, size_t off) {
-  return reinterpret_cast<T*>(reinterpret_cast<char*>(ws) + off);
+// The dense contractions of the schedule run on the tensor cores in mode 2.
+static GemmRunner gemm_runner(const seedrl_r2d2_net* n, void* ws, const RPlan& pl) {
+  return GemmRunner{n->mode >= 1, n->mode >= 2, W<float>(ws, pl.gemm_ws), W<int>(ws, pl.tcerr)};
 }
-static inline const float* RP(const seedrl_r2d2_net* n, const float* arena, int idx) {
-  return arena + n->params[idx].offset;
-}
-static inline float* RG(const seedrl_r2d2_net* n, float* arena, int idx) { return arena + n->params[idx].offset; }
-
-static int r_gemm(const seedrl_r2d2_net* n, void* ws, const RPlan& pl, bool ta, bool tb, int M, int N, int K,
-                  const float* A, int lda, const float* B, int ldb, float* C, int ldc, const GemmEpi& e,
-                  cudaStream_t st) {
-  if (n->mode >= 1 && gemm_tc_supported(M, N, K))
-    return gemm_tc(ta, tb, n->mode >= 2, M, N, K, A, lda, B, ldb, C, ldc, e, RW<float>(ws, pl.gemm_ws),
-                   gemm_tc_workspace_bytes(), RW<int>(ws, pl.tcerr), st);
-  return sgemm(ta, tb, M, N, K, A, lda, B, ldb, C, ldc, e, st);
-}
-
-// Tensor-core modes read the im2col matrix of a convolution straight from its NHWC input while the
-// GEMM stages its A blocks (kernels.h ConvGather): nothing is materialised for the forward or the
-// weight gradient.  False: geometry without aligned 8-element groups, SIMT mode, or switched off.
-static bool conv_gathered(const seedrl_r2d2_net* n, int N, const RConv& c, bool u8, const void* x, ConvGather* cg) {
-  const int K = c.k * c.k * c.cin, M = N * c.hout * c.wout;
-  return n->mode >= 1 && gemm_tc_gather_enabled() && gemm_tc_supported(M, c.cout, K) &&
-         gemm_tc_supported(K, c.cout, M) && conv_gather_setup(x, u8 ? 1 : 0, N, c.hin, c.win, c.cin, c.k, c.s, cg);
-}
-static int r_gemm_gather(const seedrl_r2d2_net* n, void* ws, const RPlan& pl, bool ta, int M, int N, int K,
-                         const ConvGather& cg, const float* B, int ldb, float* C, int ldc, const GemmEpi& e,
-                         cudaStream_t st) {
-  return gemm_tc(ta, false, n->mode >= 2, M, N, K, nullptr, 0, B, ldb, C, ldc, e, RW<float>(ws, pl.gemm_ws),
-                 gemm_tc_workspace_bytes(), RW<int>(ws, pl.tcerr), st, &cg);
-}
-
-// ------------------------------------------------------------------------------------------------
-// im2col: col[(n*Ho + ho)*Wo + wo][(kh*K + kw)*C + c] = x[n][ho*S + kh][wo*S + kw][c]  (* 1/255 for
-// uint8 frames).  Thread = VEC consecutive channels of one col element (VEC = 4 when C % 4 == 0).
-template <bool U8, int VEC>
-__global__ void __launch_bounds__(256)
-im2col_kernel(long long total, int H, int W, int C, int K, int S, int Ho, int Wo, const void* __restrict__ x_,
-              float* __restrict__ col) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total) return;
-  const int CV = C / VEC;
-  const int KK = K * K * CV;
-  const long long row = i / KK;
-  const int e = (int)(i - row * KK);
-  const int cv = e % CV, kk = e / CV, kw = kk % K, kh = kk / K;
-  const int wo = (int)(row % Wo);
-  const long long r2 = row / Wo;
-  const int ho = (int)(r2 % Ho);
-  const long long n = r2 / Ho;
-  const size_t src = (((size_t)n * H + (ho * S + kh)) * W + (wo * S + kw)) * C + (size_t)cv * VEC;
-  float* dst = col + (size_t)row * (K * K * C) + (size_t)kk * C + cv * VEC;
-  if (VEC == 4) {
-    float4 v;
-    if (U8) {
-      const uchar4 u = __ldg(reinterpret_cast<const uchar4*>(reinterpret_cast<const uint8_t*>(x_) + src));
-      const float k = 1.0f / 255.0f;
-      v = make_float4(u.x * k, u.y * k, u.z * k, u.w * k);
-    } else {
-      v = __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(x_) + src));
-    }
-    *reinterpret_cast<float4*>(dst) = v;
-  } else {
-    if (U8) *dst = (float)__ldg(reinterpret_cast<const uint8_t*>(x_) + src) * (1.0f / 255.0f);
-    else *dst = __ldg(reinterpret_cast<const float*>(x_) + src);
-  }
-}
-
-int im2col_nhwc(int N, int H, int W, int C, int K, int S, int in_u8, const void* x, float* col, cudaStream_t st) {
-  RConv c;
-  c.k = K; c.s = S; c.cin = C; c.cout = 0; c.hin = H; c.win = W; c.hout = (H - K) / S + 1; c.wout = (W - K) / S + 1;
-  c.w = c.b = 0;
-  return im2col(N, c, in_u8 != 0, x, col, st);
-}
-int col2im_nhwc(int N, int H, int W, int C, int K, int S, const float* dcol, const float* xmask, float* dx,
-                cudaStream_t st) {
-  RConv c;
-  c.k = K; c.s = S; c.cin = C; c.cout = 0; c.hin = H; c.win = W; c.hout = (H - K) / S + 1; c.wout = (W - K) / S + 1;
-  c.w = c.b = 0;
-  return col2im(N, c, dcol, xmask, dx, st);
-}
-
-static int im2col(int N, const RConv& c, bool u8, const void* x, float* col, cudaStream_t st) {
-  const int vec = (c.cin % 4 == 0) ? 4 : 1;
-  const long long total = (long long)N * c.hout * c.wout * c.k * c.k * (c.cin / vec);
-  const unsigned grid = (unsigned)((total + 255) / 256);
-#define SEEDRL_I2C(U8_, V_) \
-  im2col_kernel<U8_, V_><<<grid, 256, 0, st>>>(total, c.hin, c.win, c.cin, c.k, c.s, c.hout, c.wout, x, col)
-  if (u8) { if (vec == 4) SEEDRL_I2C(true, 4); else SEEDRL_I2C(true, 1); }
-  else    { if (vec == 4) SEEDRL_I2C(false, 4); else SEEDRL_I2C(false, 1); }
-#undef SEEDRL_I2C
-  count_launch(PC_CONV_FWD, st);
-  SEEDRL_CHECK_LAUNCH();
-  return SEEDRL_OK;
-}
-
-// col2im (gather form): dx[n][h][w][c] = sum over (kh, kw) with (h - kh) % S == 0, (w - kw) % S == 0,
-// ho = (h - kh) / S < Ho, wo < Wo of dcol[(n, ho, wo)][(kh, kw, c)], masked by x > 0 (x = the ReLU'd
-// activation this gradient flows into).  Thread = 4 channels of one input pixel.
-__global__ void __launch_bounds__(256)
-col2im_kernel(long long total, int H, int W, int C, int K, int S, int Ho, int Wo, const float* __restrict__ dcol,
-              const float* __restrict__ xmask, float* __restrict__ dx) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total) return;
-  const int C4 = C >> 2;
-  const int c4 = (int)(i % C4);
-  long long r = i / C4;
-  const int w = (int)(r % W); r /= W;
-  const int h = (int)(r % H);
-  const long long n = r / H;
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-  const int KC = K * K * C;
-  for (int kh = h % S; kh < K; kh += S) {
-    const int ho = (h - kh) / S;
-    if (h - kh < 0) break;
-    if (ho >= Ho) continue;
-    for (int kw = w % S; kw < K; kw += S) {
-      const int wo = (w - kw) / S;
-      if (w - kw < 0) break;
-      if (wo >= Wo) continue;
-      const float4 d = __ldg(reinterpret_cast<const float4*>(
-          dcol + (((size_t)n * Ho + ho) * Wo + wo) * KC + (size_t)(kh * K + kw) * C + c4 * 4));
-      acc.x += d.x; acc.y += d.y; acc.z += d.z; acc.w += d.w;
-    }
-  }
-  const float4 m = __ldg(reinterpret_cast<const float4*>(xmask) + i);
-  acc.x = m.x > 0.f ? acc.x : 0.f; acc.y = m.y > 0.f ? acc.y : 0.f;
-  acc.z = m.z > 0.f ? acc.z : 0.f; acc.w = m.w > 0.f ? acc.w : 0.f;
-  reinterpret_cast<float4*>(dx)[i] = acc;
-}
-
-static int col2im(int N, const RConv& c, const float* dcol, const float* xmask, float* dx, cudaStream_t st) {
-  const long long total = (long long)N * c.hin * c.win * (c.cin / 4);
-  col2im_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(total, c.hin, c.win, c.cin, c.k, c.s, c.hout,
-                                                                 c.wout, dcol, xmask, dx);
-  count_launch(PC_CONV_DGRAD, st);
-  SEEDRL_CHECK_LAUNCH();
-  return SEEDRL_OK;
+static LstmCore r_lstm_core(const seedrl_r2d2_net* n, void* ws, const RPlan& pl, int T, int B) {
+  return lstm_core(kRH, n->core_in, T, B, n->lstm_mode == 2, pl.lstm, ws, W<unsigned int>(ws, pl.counter));
 }
 
 // _torso tail (networks.py:262-273): core_in[n] = concat(dense_out[n] (512, already ReLU'd),
@@ -316,69 +136,62 @@ extern "C" int seedrl_r2d2_net_create(int num_actions, int obs_h, int obs_w, int
   seedrl_r2d2_net* n = new seedrl_r2d2_net();
   n->A = num_actions; n->H = obs_h; n->W = obs_w; n->C = channels;
   n->mode = 2;
-  n->arena_floats = 0;
   const int spec[3][3] = {{32, 8, 4}, {64, 4, 2}, {64, 3, 1}};     // (filters, kernel, stride) :233-238
   int h = obs_h, w = obs_w, c = channels;
   for (int i = 0; i < 3; ++i) {
-    RConv& k = n->conv[i];
-    k.k = spec[i][1]; k.s = spec[i][2]; k.cin = c; k.cout = spec[i][0];
-    k.hin = h; k.win = w; k.hout = (h - k.k) / k.s + 1; k.wout = (w - k.k) / k.s + 1;
+    StridedConv& k = n->conv[i];
+    k = strided_conv(spec[i][1], spec[i][2], c, spec[i][0], h, w);
     h = k.hout; w = k.wout; c = k.cout;
   }
   n->flat = h * w * c;
   n->core_in = kRH + 1 + num_actions;
   // tf.Module attribute order: _advantage, _body, _core, _value
-  n->p_ah_w = r_add(n, "advantage/hidden/kernel", {kRH, 512});
-  n->p_ah_b = r_add(n, "advantage/hidden/bias", {512});
-  n->p_a_w = r_add(n, "advantage/head/kernel", {512, num_actions});
+  ParamTable& pt = n->pt;
+  n->p_ah_w = pt.add("advantage/hidden/kernel", {kRH, 512});
+  n->p_ah_b = pt.add("advantage/hidden/bias", {512});
+  n->p_a_w = pt.add("advantage/head/kernel", {512, num_actions});
   for (int i = 0; i < 3; ++i) {
-    RConv& k = n->conv[i];
+    StridedConv& k = n->conv[i];
     const std::string pre = "body/conv" + std::to_string(i);
-    k.w = r_add(n, pre + "/kernel", {k.k, k.k, k.cin, k.cout});
-    k.b = r_add(n, pre + "/bias", {k.cout});
+    k.w = pt.add(pre + "/kernel", {k.k, k.k, k.cin, k.cout});
+    k.b = pt.add(pre + "/bias", {k.cout});
   }
-  n->p_dense_w = r_add(n, "body/dense/kernel", {n->flat, 512});
-  n->p_dense_b = r_add(n, "body/dense/bias", {512});
-  n->p_core_w = r_add(n, "core/kernel", {n->core_in, 4 * kRH});
-  n->p_core_u = r_add(n, "core/recurrent_kernel", {kRH, 4 * kRH});
-  n->p_core_b = r_add(n, "core/bias", {4 * kRH});
-  n->p_vh_w = r_add(n, "value/hidden/kernel", {kRH, 512});
-  n->p_vh_b = r_add(n, "value/hidden/bias", {512});
-  n->p_v_w = r_add(n, "value/head/kernel", {512, 1});
-  n->p_v_b = r_add(n, "value/head/bias", {1});
+  n->p_dense_w = pt.add("body/dense/kernel", {n->flat, 512});
+  n->p_dense_b = pt.add("body/dense/bias", {512});
+  n->p_core_w = pt.add("core/kernel", {n->core_in, 4 * kRH});
+  n->p_core_u = pt.add("core/recurrent_kernel", {kRH, 4 * kRH});
+  n->p_core_b = pt.add("core/bias", {4 * kRH});
+  n->p_vh_w = pt.add("value/hidden/kernel", {kRH, 512});
+  n->p_vh_b = pt.add("value/hidden/bias", {512});
+  n->p_v_w = pt.add("value/head/kernel", {512, 1});
+  n->p_v_b = pt.add("value/head/bias", {1});
   n->logical_params = 0;
-  for (const RParam& p : n->params) n->logical_params += p.size;
+  for (const ParamInfo& p : pt.params) n->logical_params += p.size;
   *out = n;
   return SEEDRL_OK;
 }
 
 extern "C" void seedrl_r2d2_net_destroy(seedrl_r2d2_net* net) { delete net; }
 extern "C" int seedrl_r2d2_net_num_param_tensors(const seedrl_r2d2_net* net) {
-  return net ? (int)net->params.size() : 0;
+  return net ? (int)net->pt.params.size() : 0;
 }
 extern "C" size_t seedrl_r2d2_net_num_params(const seedrl_r2d2_net* net) { return net ? net->logical_params : 0; }
-extern "C" size_t seedrl_r2d2_net_arena_floats(const seedrl_r2d2_net* net) { return net ? net->arena_floats : 0; }
+extern "C" size_t seedrl_r2d2_net_arena_floats(const seedrl_r2d2_net* net) { return net ? net->pt.arena_floats : 0; }
 extern "C" int seedrl_r2d2_net_set_mode(seedrl_r2d2_net* net, int mode) {
   SEEDRL_CHECK_ARG(net && (mode == 0 || mode == 2), "mode must be 0 (fp32 SIMT) or 2 (tcgen05 bf16x3)");
   net->mode = mode;
   return SEEDRL_OK;
 }
 extern "C" int seedrl_r2d2_net_set_lstm_mode(seedrl_r2d2_net* net, int mode) {
-  SEEDRL_CHECK_ARG(net && (mode == 1 || mode == 2), "mode must be 1 (persistent) or 2 (tiled persistent)");
+  SEEDRL_CHECK_ARG(net && (mode == 0 || mode == 2), "mode must be 0 (per-step launches) or 2 (tiled persistent)");
   net->lstm_mode = mode;
   return SEEDRL_OK;
 }
 extern "C" int seedrl_r2d2_net_param_info(const seedrl_r2d2_net* net, int index, char* name_buf, size_t name_cap,
                                           int64_t* dims4, int* rank, size_t* offset_floats) {
-  SEEDRL_CHECK_ARG(net && index >= 0 && index < (int)net->params.size(), "bad index");
-  const RParam& p = net->params[index];
-  if (name_buf && name_cap) {
-    strncpy(name_buf, p.name.c_str(), name_cap - 1);
-    name_buf[name_cap - 1] = 0;
-  }
-  if (dims4) for (int i = 0; i < 4; ++i) dims4[i] = p.dims[i];
-  if (rank) *rank = p.rank;
-  if (offset_floats) *offset_floats = p.offset;
+  SEEDRL_CHECK_ARG(net && index >= 0 && index < (int)net->pt.params.size(), "bad index");
+  const int r = net->pt.info(index, name_buf, name_cap, dims4, offset_floats);
+  if (rank) *rank = r;
   return SEEDRL_OK;
 }
 extern "C" size_t seedrl_r2d2_net_workspace_bytes(const seedrl_r2d2_net* net, int T, int B) {
@@ -400,63 +213,43 @@ extern "C" int seedrl_r2d2_net_forward(const seedrl_r2d2_net* n, const float* pr
                    "unroll batch too large (GEMM row count)");
   cudaStream_t st = (cudaStream_t)stream;
   const int N = (int)pl.N, A = n->A, CI = n->core_in;
-  SEEDRL_CUDA(cudaMemsetAsync(RW<int>(ws, pl.tcerr), 0, sizeof(int), st));
-  // ---- body: three convolutions as im2col + GEMM (bias + ReLU in the epilogue) ----------------
+  const ParamTable& pt = n->pt;
+  const GemmRunner g = gemm_runner(n, ws, pl);
+  SEEDRL_CUDA(cudaMemsetAsync(g.err, 0, sizeof(int), st));
+  // ---- body: three strided convolutions (bias + ReLU in the GEMM epilogue) ----------------------
   const void* x = frames;
   for (int i = 0; i < 3; ++i) {
-    const RConv& c = n->conv[i];
-    float* col = RW<float>(ws, pl.col[i]);
-    float* act = RW<float>(ws, pl.act[i]);
-    GemmEpi e = epi_none();
-    e.bias = RP(n, prm, c.b); e.relu = 1;
-    const int K = c.k * c.k * c.cin;
-    ConvGather cg;
-    if (conv_gathered(n, N, c, i == 0, x, &cg)) {
-      SEEDRL_TRY(r_gemm_gather(n, ws, pl, false, N * c.hout * c.wout, c.cout, K, cg, RP(n, prm, c.w), c.cout, act,
-                               c.cout, e, st));
-    } else {
-      SEEDRL_TRY(im2col(N, c, i == 0, x, col, st));
-      SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N * c.hout * c.wout, c.cout, K, col, K, RP(n, prm, c.w), c.cout,
-                        act, c.cout, e, st));
-    }
+    const StridedConv& c = n->conv[i];
+    float* act = W<float>(ws, pl.act[i]);
+    SEEDRL_TRY(strided_conv_forward(g, N, c, i == 0, x, pt.at(prm, c.w), pt.at(prm, c.b), W<float>(ws, pl.col[i]),
+                                    act, st));
     x = act;
   }
-  float* xc = RW<float>(ws, pl.xc); float* z = RW<float>(ws, pl.z);
-  float* hp = RW<float>(ws, pl.hp); float* cs = RW<float>(ws, pl.cs); float* hs = RW<float>(ws, pl.hs);
-  float* c0buf = RW<float>(ws, pl.c0buf);
+  const LstmCore core = r_lstm_core(n, ws, pl, T, B);
+  float* xc = core.xc; float* hs = core.hs; float* cs = core.cs;
   // Flatten (NHWC order) + Dense(512) + ReLU written into the first 512 columns of the core input
   GemmEpi e = epi_none();
-  e.bias = RP(n, prm, n->p_dense_b); e.relu = 1;
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N, kRH, n->flat, RW<float>(ws, pl.act[2]), n->flat,
-                    RP(n, prm, n->p_dense_w), kRH, xc, CI, e, st));
+  e.bias = pt.at(prm, n->p_dense_b); e.relu = 1;
+  SEEDRL_TRY(g.gemm(false, false, N, kRH, n->flat, W<float>(ws, pl.act[2]), n->flat, pt.at(prm, n->p_dense_w), kRH,
+                    xc, CI, e, st));
   r2d2_core_tail_kernel<<<ceil_div(N * (1 + A), 256), 256, 0, st>>>(N, kRH, A, reward, prev_actions, xc);
   count_launch(PC_MISC, st);
   SEEDRL_CHECK_LAUNCH();
-  // LSTM input projection for all T at once, then the persistent recurrence
-  e = epi_none();
-  e.bias = RP(n, prm, n->p_core_b);
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N, 4 * kRH, CI, xc, CI, RP(n, prm, n->p_core_w), 4 * kRH, z, 4 * kRH, e,
-                    st));
-  SEEDRL_CUDA(cudaMemcpyAsync(c0buf, c0, (size_t)B * kRH * 4, cudaMemcpyDeviceToDevice, st));
-  if (n->lstm_mode == 2)
-    SEEDRL_TRY(lstm_forward_tiled(kRH, T, B, RP(n, prm, n->p_core_u), done, z, h0, c0buf, hs, cs, hp,
-                                  RW<unsigned int>(ws, pl.counter), RW<int>(ws, pl.tcerr), st));
-  else
-    SEEDRL_TRY(lstm_forward_persistent(kRH, T, B, RP(n, prm, n->p_core_u), done, z, h0, c0buf, hs, cs, hp,
-                                       RW<unsigned int>(ws, pl.counter), RW<int>(ws, pl.tcerr), st));
+  SEEDRL_TRY(lstm_core_forward(g, core, pt.at(prm, n->p_core_w), pt.at(prm, n->p_core_u), pt.at(prm, n->p_core_b),
+                               done, h0, c0, st));
   // dueling heads
-  float* vh = RW<float>(ws, pl.vh); float* ah = RW<float>(ws, pl.ah);
-  float* v = RW<float>(ws, pl.v); float* adv = RW<float>(ws, pl.adv);
+  float* vh = W<float>(ws, pl.vh); float* ah = W<float>(ws, pl.ah);
+  float* v = W<float>(ws, pl.v); float* adv = W<float>(ws, pl.adv);
   e = epi_none();
-  e.bias = RP(n, prm, n->p_vh_b); e.relu = 1;
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N, 512, kRH, hs, kRH, RP(n, prm, n->p_vh_w), 512, vh, 512, e, st));
-  e.bias = RP(n, prm, n->p_ah_b);
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N, 512, kRH, hs, kRH, RP(n, prm, n->p_ah_w), 512, ah, 512, e, st));
+  e.bias = pt.at(prm, n->p_vh_b); e.relu = 1;
+  SEEDRL_TRY(g.gemm(false, false, N, 512, kRH, hs, kRH, pt.at(prm, n->p_vh_w), 512, vh, 512, e, st));
+  e.bias = pt.at(prm, n->p_ah_b);
+  SEEDRL_TRY(g.gemm(false, false, N, 512, kRH, hs, kRH, pt.at(prm, n->p_ah_w), 512, ah, 512, e, st));
   e = epi_none();
-  e.bias = RP(n, prm, n->p_v_b);
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N, 1, 512, vh, 512, RP(n, prm, n->p_v_w), 1, v, 1, e, st));
+  e.bias = pt.at(prm, n->p_v_b);
+  SEEDRL_TRY(g.gemm(false, false, N, 1, 512, vh, 512, pt.at(prm, n->p_v_w), 1, v, 1, e, st));
   e = epi_none();
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, false, N, A, 512, ah, 512, RP(n, prm, n->p_a_w), A, adv, A, e, st));
+  SEEDRL_TRY(g.gemm(false, false, N, A, 512, ah, 512, pt.at(prm, n->p_a_w), A, adv, A, e, st));
   dueling_fwd_kernel<<<ceil_div(N, 128), 128, 0, st>>>(N, A, v, adv, q_values, action);
   count_launch(PC_MISC, st);
   SEEDRL_CHECK_LAUNCH();
@@ -477,15 +270,15 @@ extern "C" int seedrl_r2d2_net_backward(const seedrl_r2d2_net* n, const float* p
   const RPlan pl = r_plan(n, T, B);
   SEEDRL_CHECK_ARG(ws_bytes >= pl.total, "workspace too small");
   cudaStream_t st = (cudaStream_t)stream;
-  const int N = (int)pl.N, A = n->A, CI = n->core_in;
-  float* xc = RW<float>(ws, pl.xc); float* z = RW<float>(ws, pl.z);
-  float* hp = RW<float>(ws, pl.hp); float* cs = RW<float>(ws, pl.cs); float* hs = RW<float>(ws, pl.hs);
-  float* c0buf = RW<float>(ws, pl.c0buf);
-  float* vh = RW<float>(ws, pl.vh); float* ah = RW<float>(ws, pl.ah);
-  float* dv = RW<float>(ws, pl.dv); float* dadv = RW<float>(ws, pl.dadv);
-  float* dvh = RW<float>(ws, pl.dvh); float* dah = RW<float>(ws, pl.dah);
-  float* dhs = RW<float>(ws, pl.dhs); float* dz = RW<float>(ws, pl.dz); float* dd = RW<float>(ws, pl.dd);
-  SEEDRL_CUDA(cudaMemsetAsync(grd, 0, n->arena_floats * sizeof(float), st));
+  const int N = (int)pl.N, A = n->A;
+  const ParamTable& pt = n->pt;
+  const GemmRunner g = gemm_runner(n, ws, pl);
+  const LstmCore core = r_lstm_core(n, ws, pl, T, B);
+  float* hs = core.hs; float* dhs = core.dhs; float* dd = core.dd;
+  float* vh = W<float>(ws, pl.vh); float* ah = W<float>(ws, pl.ah);
+  float* dv = W<float>(ws, pl.dv); float* dadv = W<float>(ws, pl.dadv);
+  float* dvh = W<float>(ws, pl.dvh); float* dah = W<float>(ws, pl.dah);
+  SEEDRL_CUDA(cudaMemsetAsync(grd, 0, pt.arena_floats * sizeof(float), st));
   const GemmEpi e0 = epi_none();
   GemmEpi eacc = epi_none();
   eacc.accumulate = 1;
@@ -494,63 +287,37 @@ extern "C" int seedrl_r2d2_net_backward(const seedrl_r2d2_net* n, const float* p
   count_launch(PC_MISC, st);
   SEEDRL_CHECK_LAUNCH();
   // advantage stream
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, 512, A, N, ah, 512, dadv, A, RG(n, grd, n->p_a_w), A, e0, st));
+  SEEDRL_TRY(g.gemm(true, false, 512, A, N, ah, 512, dadv, A, pt.at(grd, n->p_a_w), A, e0, st));
   GemmEpi em = epi_none();
   em.mask = ah; em.ldm = 512;
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, true, N, 512, A, dadv, A, RP(n, prm, n->p_a_w), A, dah, 512, em, st));
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, kRH, 512, N, hs, kRH, dah, 512, RG(n, grd, n->p_ah_w), 512, e0, st));
-  SEEDRL_TRY(colsum(N, 512, dah, 512, RG(n, grd, n->p_ah_b), st, RW<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
+  SEEDRL_TRY(g.gemm(false, true, N, 512, A, dadv, A, pt.at(prm, n->p_a_w), A, dah, 512, em, st));
+  SEEDRL_TRY(g.gemm(true, false, kRH, 512, N, hs, kRH, dah, 512, pt.at(grd, n->p_ah_w), 512, e0, st));
+  SEEDRL_TRY(g.colsum(N, 512, dah, 512, pt.at(grd, n->p_ah_b), st));
   // value stream
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, 512, 1, N, vh, 512, dv, 1, RG(n, grd, n->p_v_w), 1, e0, st));
-  SEEDRL_TRY(colsum(N, 1, dv, 1, RG(n, grd, n->p_v_b), st, RW<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
+  SEEDRL_TRY(g.gemm(true, false, 512, 1, N, vh, 512, dv, 1, pt.at(grd, n->p_v_w), 1, e0, st));
+  SEEDRL_TRY(g.colsum(N, 1, dv, 1, pt.at(grd, n->p_v_b), st));
   em.mask = vh;
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, true, N, 512, 1, dv, 1, RP(n, prm, n->p_v_w), 1, dvh, 512, em, st));
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, kRH, 512, N, hs, kRH, dvh, 512, RG(n, grd, n->p_vh_w), 512, e0, st));
-  SEEDRL_TRY(colsum(N, 512, dvh, 512, RG(n, grd, n->p_vh_b), st, RW<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
+  SEEDRL_TRY(g.gemm(false, true, N, 512, 1, dv, 1, pt.at(prm, n->p_v_w), 1, dvh, 512, em, st));
+  SEEDRL_TRY(g.gemm(true, false, kRH, 512, N, hs, kRH, dvh, 512, pt.at(grd, n->p_vh_w), 512, e0, st));
+  SEEDRL_TRY(g.colsum(N, 512, dvh, 512, pt.at(grd, n->p_vh_b), st));
   // d core output
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, true, N, kRH, 512, dah, 512, RP(n, prm, n->p_ah_w), 512, dhs, kRH, e0, st));
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, true, N, kRH, 512, dvh, 512, RP(n, prm, n->p_vh_w), 512, dhs, kRH, eacc, st));
-  // BPTT
-  if (n->lstm_mode == 2)
-    SEEDRL_TRY(lstm_backward_tiled(kRH, T, B, RP(n, prm, n->p_core_u), done, z, cs, c0buf, dhs, dz,
-                                   RW<unsigned int>(ws, pl.counter), RW<int>(ws, pl.tcerr), st));
-  else
-    SEEDRL_TRY(lstm_backward_persistent(kRH, T, B, RP(n, prm, n->p_core_u), done, z, cs, c0buf, dhs, dz,
-                                        RW<unsigned int>(ws, pl.counter), RW<int>(ws, pl.tcerr), st));
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, kRH, 4 * kRH, N, hp, kRH, dz, 4 * kRH, RG(n, grd, n->p_core_u), 4 * kRH,
-                    e0, st));
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, CI, 4 * kRH, N, xc, CI, dz, 4 * kRH, RG(n, grd, n->p_core_w), 4 * kRH, e0,
-                    st));
-  SEEDRL_TRY(colsum(N, 4 * kRH, dz, 4 * kRH, RG(n, grd, n->p_core_b), st, RW<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-  // d dense_out = (dz W[:512,:]^T) * (dense_out > 0)
-  em.mask = xc; em.ldm = CI;
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, true, N, kRH, 4 * kRH, dz, 4 * kRH, RP(n, prm, n->p_core_w), 4 * kRH, dd, kRH,
-                    em, st));
-  const float* flat = RW<float>(ws, pl.act[2]);
-  SEEDRL_TRY(r_gemm(n, ws, pl, true, false, n->flat, kRH, N, flat, n->flat, dd, kRH, RG(n, grd, n->p_dense_w), kRH,
-                    e0, st));
-  SEEDRL_TRY(colsum(N, kRH, dd, kRH, RG(n, grd, n->p_dense_b), st, RW<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
+  SEEDRL_TRY(g.gemm(false, true, N, kRH, 512, dah, 512, pt.at(prm, n->p_ah_w), 512, dhs, kRH, e0, st));
+  SEEDRL_TRY(g.gemm(false, true, N, kRH, 512, dvh, 512, pt.at(prm, n->p_vh_w), 512, dhs, kRH, eacc, st));
+  SEEDRL_TRY(lstm_core_backward(g, core, pt.at(prm, n->p_core_w), pt.at(prm, n->p_core_u), done,
+                                pt.at(grd, n->p_core_w), pt.at(grd, n->p_core_u), pt.at(grd, n->p_core_b), st));
+  const float* flat = W<float>(ws, pl.act[2]);
+  SEEDRL_TRY(g.gemm(true, false, n->flat, kRH, N, flat, n->flat, dd, kRH, pt.at(grd, n->p_dense_w), kRH, e0, st));
+  SEEDRL_TRY(g.colsum(N, kRH, dd, kRH, pt.at(grd, n->p_dense_b), st));
   em.mask = flat; em.ldm = n->flat;
-  SEEDRL_TRY(r_gemm(n, ws, pl, false, true, N, n->flat, kRH, dd, kRH, RP(n, prm, n->p_dense_w), kRH,
-                    RW<float>(ws, pl.g[2]), n->flat, em, st));
-  // convolutions, last to first
+  SEEDRL_TRY(g.gemm(false, true, N, n->flat, kRH, dd, kRH, pt.at(prm, n->p_dense_w), kRH, W<float>(ws, pl.g[2]),
+                    n->flat, em, st));
+  // convolutions, last to first; no gradient flows into the frames
   for (int i = 2; i >= 0; --i) {
-    const RConv& c = n->conv[i];
-    const int K = c.k * c.k * c.cin, M = N * c.hout * c.wout;
-    float* col = RW<float>(ws, pl.col[i]);
-    const float* g = RW<float>(ws, pl.g[i]);
-    // weight gradient = im2col(input)^T g: gathered from the layer's input, or from the matrix the forward kept
-    const void* xin = i == 0 ? (const void*)frames : (const void*)RW<float>(ws, pl.act[i - 1]);
-    ConvGather cg;
-    if (conv_gathered(n, N, c, i == 0, xin, &cg))
-      SEEDRL_TRY(r_gemm_gather(n, ws, pl, true, K, c.cout, M, cg, g, c.cout, RG(n, grd, c.w), c.cout, e0, st));
-    else
-      SEEDRL_TRY(r_gemm(n, ws, pl, true, false, K, c.cout, M, col, K, g, c.cout, RG(n, grd, c.w), c.cout, e0, st));
-    SEEDRL_TRY(colsum(M, c.cout, g, c.cout, RG(n, grd, c.b), st, RW<float>(ws, pl.gemm_ws), gemm_tc_workspace_bytes()));
-    if (i > 0) {
-      SEEDRL_TRY(r_gemm(n, ws, pl, false, true, M, K, c.cout, g, c.cout, RP(n, prm, c.w), c.cout, col, K, e0, st));
-      SEEDRL_TRY(col2im(N, c, col, RW<float>(ws, pl.act[i - 1]), RW<float>(ws, pl.g[i - 1]), st));
-    }
+    const StridedConv& c = n->conv[i];
+    const void* xin = i == 0 ? (const void*)frames : (const void*)W<float>(ws, pl.act[i - 1]);
+    SEEDRL_TRY(strided_conv_backward(g, N, c, i == 0, xin, W<float>(ws, pl.col[i]), pt.at(prm, c.w),
+                                     W<float>(ws, pl.g[i]), pt.at(grd, c.w), pt.at(grd, c.b),
+                                     i > 0 ? W<float>(ws, pl.g[i - 1]) : nullptr, st));
   }
   return SEEDRL_OK;
 }
@@ -560,12 +327,5 @@ extern "C" int seedrl_r2d2_net_check_error(const seedrl_r2d2_net* n, int T, int 
   SEEDRL_CHECK_ARG(n && ws && T >= 1 && B >= 1, "bad arguments");
   const RPlan pl = r_plan(n, T, B);
   SEEDRL_CHECK_ARG(ws_bytes >= pl.total, "workspace too small");
-  int flag = 0;
-  SEEDRL_CUDA(cudaMemcpyAsync(&flag, RW<int>(ws, pl.tcerr), sizeof(int), cudaMemcpyDeviceToHost,
-                              (cudaStream_t)stream));
-  SEEDRL_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-  if (flag != 0)
-    return set_error(SEEDRL_ERR_INTERNAL,
-                     "a tensor-core / persistent kernel timed out on a barrier: results of this unroll are invalid");
-  return SEEDRL_OK;
+  return read_error_flag(W<int>(ws, pl.tcerr), (cudaStream_t)stream);
 }

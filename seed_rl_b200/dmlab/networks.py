@@ -52,9 +52,9 @@ class _CudaAgent(object):
       raise ValueError("conv_mode 'tc3p' is built for the deep net")
     self.conv_mode = conv_mode
     _lib.check(L.seedrl_net_set_conv_mode(h, modes[conv_mode]))
-    lstm_modes = {'stepwise': 0, 'persistent': 1, 'tiled': 2}
+    lstm_modes = {'stepwise': 0, 'tiled': 2}
     if lstm_mode not in lstm_modes:
-      raise ValueError("lstm_mode must be 'tiled', 'persistent' or 'stepwise'")
+      raise ValueError("lstm_mode must be 'tiled' or 'stepwise'")
     self.lstm_mode = lstm_mode
     _lib.check(L.seedrl_net_set_lstm_mode(h, lstm_modes[lstm_mode]))
     self._n_tensors = L.seedrl_net_num_param_tensors(h)

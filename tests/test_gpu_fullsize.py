@@ -7,8 +7,8 @@ agents/vtrace/learner.py:73-159,255-280 + dmlab/networks.py:26-171) at
   * T=20, B=256 (cfg 3): forward outputs and final LSTM state.
 
 At these sizes the 512-position conv tiles wrap many frames, split-K runs all its splits, the
-deferred weight-gradient partial buffer is full and the persistent LSTM runs all 21 grid
-barriers -- the toy-size tests in test_gpu_parity.py exercise none of that.
+deferred weight-gradient partial buffer is full and the tiled LSTM runs all 21 steps behind
+its per-tile barriers -- the toy-size tests in test_gpu_parity.py exercise none of that.
 
 Tolerances (stated, per mode):
   forward outputs   2e-4 of the tensor's max-abs (+2e-5 abs)

@@ -81,34 +81,3 @@ def test_shallow_net_gathered_equals_materialised(mode, T, B):
     assert torch.equal(x, y)
   assert float(r[1][1].abs().max()) > 0
 
-
-@pytest.mark.parametrize('T,B', [(5, 40), (3, 64), (4, 9), (2, 100)])
-def test_r2d2_lstm512_tiled_matches_first_form(T, B):
-  """LSTM(512) recurrence of the R2D2 net (atari/networks.py:240-252): the tiled kernel (batch tiles of
-  8 / 16 / 32 rows chosen so that tiles x 32 unit groups stay co-resident) against the first persistent
-  form (CTA = 4 units x all rows), same fp32 arithmetic, different summation order."""
-  from oracle import r2d2_learner_oracle as RL
-  from seed_rl_b200 import _lib
-  from seed_rl_b200.atari import networks
-  from seed_rl_b200.common import utils
-  A, obs, S = 6, (36, 36, 1), 4
-  b = RL.synthetic_replay_batch(T, B, A, obs, seed=B, done_p=0.2)
-  c = lambda a: torch.as_tensor(np.asarray(a)).cuda()
-  env = utils.EnvOutput(c(b['reward']), c(b['done']), c(b['observation']),
-                        torch.zeros(T, B, dtype=torch.bool).cuda(), torch.zeros(T, B, dtype=torch.int32).cuda())
-  state = networks.AgentState((c(b['h0']), c(b['c0'])), c(b['frame_state']))
-  agent = networks.DuelingLSTMDQNNet(A, obs, S, seed=11, gemm_mode='tc3')
-  dq = torch.randn(T, B, A, device='cuda', generator=torch.Generator(device='cuda').manual_seed(2))
-  res = {}
-  for mode in (2, 1):
-    _lib.check(_lib.lib().seedrl_r2d2_net_set_lstm_mode(agent._h, mode))
-    out, st = agent((c(b['prev_actions']), env), state, unroll=True, is_training=True)
-    agent.backward(dq)
-    agent.check_errors()
-    res[mode] = (out.q_values.clone(), st.core_state[0].clone(), st.core_state[1].clone(), agent.grads.clone())
-  for x, y in zip(res[2][:3], res[1][:3]):
-    scale = float(y.abs().max()) + 1e-30
-    assert float((x - y).abs().max()) <= 2e-5 * scale, float((x - y).abs().max()) / scale
-  # gradients: L2 (a head unit within rounding of its ReLU kink may flip between the two summation orders)
-  gx, gy = res[2][3].double(), res[1][3].double()
-  assert float((gx - gy).norm() / gy.norm()) <= 1e-4

@@ -79,41 +79,6 @@ def test_inference_unrolls_are_consistent_with_training_unroll():
   assert host.unroll_queue.size() == 2
 
 
-@pytest.mark.parametrize('T,B', [(6, 5), (3, 70), (1, 3), (20, 64), (5, 256), (4, 300)])
-def test_persistent_lstm_matches_stepwise_schedule(T, B):
-  """The cooperative persistent-LSTM kernels (one launch for all T steps, each way) against
-  the per-step GEMM + pointwise schedule: same logits, state and gradients (fp32, different
-  summation order => 1e-5 / 1e-4)."""
-  from oracle import learner_oracle
-  from seed_rl_b200.agents.vtrace import learner
-  from seed_rl_b200.common import optimizers
-  from seed_rl_b200.dmlab import networks
-  from test_gpu_parity import _batch_to_cuda
-  b = learner_oracle.synthetic_batch(T, B, A, seed=5)
-  b['done'][min(1, T), 0] = True
-  rng = np.random.default_rng(1)
-  b['h0'] = rng.normal(size=b['h0'].shape).astype(np.float32)
-  b['c0'] = rng.normal(size=b['c0'].shape).astype(np.float32)
-  u = _batch_to_cuda(b)
-  res = {}
-  for mode in ('stepwise', 'persistent', 'tiled'):
-    agent = networks.ImpalaShallow(A, OBS, seed=2, lstm_mode=mode)    # cheap torso, same LSTM
-    step = learner.LearnerStep(agent, optimizers.Adam(1e-3))
-    out, (h, c) = agent(u.prev_actions, u.env_outputs, u.agent_state, unroll=True)
-    loss, _ = step.compute_gradients(u)
-    res[mode] = (out.policy_logits.clone(), h.clone(), c.clone(), float(loss),
-                 {k: v.clone() for k, v in agent.named_gradients().items()})
-  a = res['stepwise']
-  for name in ('persistent', 'tiled'):       # lstm_persistent.cu / lstm_tiled.cu (the default)
-    p = res[name]
-    for i in range(3):
-      np.testing.assert_allclose(p[i].cpu().numpy(), a[i].cpu().numpy(), rtol=1e-5, atol=1e-5, err_msg=name)
-    assert abs(a[3] - p[3]) < 1e-5 * max(1.0, abs(a[3])), name
-    for k in a[4]:
-      x, y = p[4][k].cpu().numpy(), a[4][k].cpu().numpy()
-      assert np.abs(x - y).max() <= 1e-4 * (np.abs(y).max() + 1e-12), (name, k)
-
-
 class _OneShot(object):
   def __init__(self, u):
     self.u = u
